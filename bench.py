@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--codec hsq|qsgd|terngrad|sign|topk] [--k-bit 8|12] [--c-dim 8|16|32] [--n-bit n]
-                    [--cr 100] [--mode ps|ring] [--workload resnet50|flat]
+                    [--cr 100] [--mode ps|ring] [--workload resnet50|flat] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default (the headline, BASELINE.json configs[1]): the 161 gradient tensors of the reference's CIFAR
@@ -19,6 +19,11 @@ on both sides, max over ranks; inputs rotate over buffers larger than L2.
 --impl reference: the same workload through the reference's CPU path on the host cores (the
 C/OpenMP oracle port with every host thread; rank 0 only), and -- when baseline/_ref is staged --
 the UNMODIFIED Python reference (baseline/ref_runner.py) beside it as `reference_py_value`.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the gradient its last timed step handed back
+(every tensor flattened, concatenated in model order, float32) as DIR/gradient.npy.  Larger outputs are
+cut to a fixed seeded sample of DUMP_MAX_ELEMS positions (see dump_outputs()).  The inputs depend only
+on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -29,6 +34,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -55,7 +61,11 @@ def parse_args():
     ap.add_argument("--sign-wire", type=str, default="2bit", choices=["2bit", "t5"],
                     help="SignSGD wire container: 2 bits per element, or base 3 with five elements per byte")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write the gradient of the last timed step to DIR/gradient.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     d = CODEC_DEFAULTS[a.codec]
     if a.c_dim is None:
         a.c_dim = d["c_dim"]
@@ -156,6 +166,22 @@ def measured_peaks():
         with open(path) as fh:
             return json.load(fh), "measured"
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}, "fallback"
+
+
+DUMP_MAX_ELEMS = 8 * 1024 * 1024         # 32 MB of float32 per dump
+
+
+def dump_outputs(out_dir, flat):
+    """--dump-outputs: write `flat` (the step's gradient in model order) as out_dir/gradient.npy, float32.
+    Above DUMP_MAX_ELEMS elements only a sample is written: the elements at the sorted positions
+    np.random.RandomState(0).choice(n, DUMP_MAX_ELEMS, replace=False).  The sample depends on n alone,
+    so it is the same in every build."""
+    import numpy as np
+    flat = np.asarray(flat, dtype=np.float32).reshape(-1)
+    if flat.size > DUMP_MAX_ELEMS:
+        flat = flat[np.sort(np.random.RandomState(0).choice(flat.size, DUMP_MAX_ELEMS, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "gradient.npy"), flat)
 
 
 # ------------------------------------------------------------------ clocks ---
@@ -349,14 +375,15 @@ class CpuPort:
                 self.codecs.append(O.TopK(n, s, a.cr))
         self.draws = rs.random_sample(n_draws * n_users).astype(np.float32)
         self.elems = sum(sizes) * n_users
+        self.out = None
 
     def step(self):
         O = self.O
         t0 = time.perf_counter()
         if self.a.mode == "ps":
-            O.ps_step(self.codecs, self.grads, O.UniformStream(self.draws))
+            self.out = O.ps_step(self.codecs, self.grads, O.UniformStream(self.draws))
         else:
-            O.ring_step(self.codecs, self.grads, O.UniformStream(self.draws))
+            self.out = O.ring_step(self.codecs, self.grads, O.UniformStream(self.draws))
         return time.perf_counter() - t0
 
 
@@ -401,6 +428,8 @@ def run_reference_arm(a):
         done_w += 1
     k_eff = K if t_first * K < budget else max(int(budget / max(t_first, 1e-6)), 1)
     times = [port.step() for _ in range(k_eff)]
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, np.concatenate([o.reshape(-1) for o in port.out]))
     t = float(np.mean(times))
     value = port.elems / t
     ref_py = reference_python(a, n_users, steps=1 if n_users > 2 else 2, warmup=1)
@@ -446,9 +475,12 @@ def main():
     numa = bind_to_gpu_numa(local_rank)
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
+    # torch seeds its default generators at random in every process; the stochastic-rounding draws
+    # (Philox keyed by the CUDA generator's seed, mixed with the user) must be the same in every run
+    torch.manual_seed(1)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    W, K = max(a.warmup, 3), max(a.steps, 1)
+    W, K = max(a.warmup, 3), a.steps
 
     shapes = workload_shapes(a.workload)
     args = make_args(a, world)
@@ -505,6 +537,10 @@ def main():
     barrier()
     ms_per_step = all_max(e0.elapsed_time(e1)) / K
     value = world * n_total / (ms_per_step * 1e-3)
+    if a.dump_outputs and rank == 0:
+        # the buffer of the last timed step, before the per-kernel and end-to-end loops below reuse it
+        last = plan.views(outputs[(K - 1) % ROT])
+        dump_outputs(a.dump_outputs, torch.cat([v.reshape(-1) for v in last]).cpu().numpy())
 
     # ---- per-kernel timing (same rotation; every rank runs them, rank 0 reports) ----
     def time_loop(fn, iters):
