@@ -30,12 +30,14 @@ class ProbabilisticScalarCompressor(object):
         seg = single_segment(n, dev)
         random = 1 if self.random else 0
         r = uniforms_arg(uniforms, n, dev) if random else None
-        if random and r is None and self.rng == "torch":
-            # reference-faithful draw: CPU generator, skipped when lb == ub (:15-16, :23-25)
+        torch_rng = random and r is None and self.rng == "torch"
+        if torch_rng:
+            # reference-faithful draw: CPU generator, skipped when lb == ub (:15-16, :23-25); the levels
+            # are then all 0 whatever the draws, so the Philox stream is not touched either
             lo, hi = torch.aminmax(v)
             if (lo - hi).item() != 0.0:
                 r = torch.rand(n).to(dev)
-        seed, off = _lib.PHILOX.take(n) if (random and r is None) else (0, 0)
+        seed, off = _lib.PHILOX.take(n) if (random and r is None and not torch_rng) else (0, 0)
         _lib.call("gq_norm_quantize", _lib.ptr(v), n, _lib.ptr(seg), 1, self.n_bit, random, _lib.ptr(r),
                   seed, off, _lib.ptr(l), 4, _lib.ptr(lbub), _lib.ptr(keys), 0, _lib.stream())
         return lbub[0], lbub[1], l.view(vec.shape)
