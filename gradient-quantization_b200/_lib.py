@@ -35,6 +35,11 @@ _SIGNATURES = {
     "gq_hsq_decode_reduce": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_i64, c_int,
                                      c_i64, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int,
                                      c_void_p, c_void_p]),
+    "gq_hsq_encode_search": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int,
+                                     c_void_p, c_void_p, c_size, c_void_p]),
+    "gq_hsq_decode_quantize": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_int, c_void_p,
+                                       c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_u64, c_u64, c_int,
+                                       c_void_p, c_void_p]),
     "gq_hsq_decode_reduce_scattered": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_i64,
                                                c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int,
                                                c_void_p, c_void_p]),

@@ -283,6 +283,62 @@ int gq_hsq_encode(const float *grad, int64_t n_chunks, int d, const float *codeb
                             philox_offset, l, l_bytes, lbub, keys, /*precomputed=*/1, stream);
 }
 
+int gq_hsq_encode_search(const float *grad, int64_t n_chunks, int d, const float *codebook, int K,
+                         const int64_t *seg_start, int n_seg, void *codes, int code_bytes, float *u_out,
+                         void *workspace, size_t workspace_bytes, gq_stream_t stream)
+{
+    const Rider rider = take_rider();
+    const Tc2Remote remote = take_remote();
+    GQ_REQUIRE(remote.n == 0, "a remote delivery needs the levels: use gq_hsq_encode");
+    int e = validate_group(grad, n_chunks, d, codebook, K, seg_start, n_seg);
+    if (e) return e;
+    const size_t need = gq_hsq_encode_workspace_bytes(n_chunks, d, K, n_seg);
+    if (workspace_bytes < need || workspace == nullptr) {
+        set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+        return GQ_ERR_WORKSPACE;
+    }
+    GQ_REQUIRE(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
+    GQ_REQUIRE(codes && u_out, "null output pointer");
+    if (tc_generation() != 2 || n_chunks == 0 || !hsq_tc2_supported(d, K, code_bytes)) {
+        set_error("gq_hsq_encode_search runs the second-generation tcgen05 search only (d in {8, 16, 32}, K == 256, "
+                  "uint8 codes, n_chunks > 0); got d=%d K=%d code_bytes=%d n_chunks=%lld",
+                  d, K, code_bytes, (long long)n_chunks);
+        return GQ_ERR_UNSUPPORTED;
+    }
+    uint32_t *keys = reinterpret_cast<uint32_t *>(workspace);
+    uint32_t *barrier = reinterpret_cast<uint32_t *>((char *)workspace + align_up((size_t)n_seg * 2 * sizeof(uint32_t), 256));
+    return hsq_encode_tc2(grad, n_chunks, d, codebook, codes, u_out, seg_start, n_seg, keys,
+                          reinterpret_cast<uint64_t *>(barrier) + 1, nullptr, rider, nullptr, nullptr, as_stream(stream));
+}
+
+static const int64_t kStageChunks = 1024;   // chunk indices of the last tile stay below 2^31
+int gq_hsq_decode_quantize(const void *codes, void *l, float *lbub, const float *u, const uint32_t *minmax_keys,
+                           int64_t n_chunks, int d, const float *codebook, int K, const int64_t *seg_start,
+                           int n_seg, int n_bit, int random, const float *uniforms, uint64_t philox_seed,
+                           uint64_t philox_offset, int accumulate, float *out, gq_stream_t stream)
+{
+    const Rider pending = take_rider();   // consumed first: an early error return must not leave it armed
+    int e = validate_group(out, n_chunks, d, codebook, K, seg_start, n_seg);
+    if (e) return e;
+    if (d != 16 || K != 256 || n_chunks == 0 || n_chunks >= ((int64_t)1 << 31) - kStageChunks || n_seg > 1024) {
+        set_error("gq_hsq_decode_quantize: d == 16, K == 256, 1 <= n_seg <= 1024, 0 < n_chunks < 2^31 - 1024 "
+                  "(got d=%d K=%d n_seg=%d n_chunks=%lld)", d, K, n_seg, (long long)n_chunks);
+        return GQ_ERR_UNSUPPORTED;
+    }
+    GQ_REQUIRE(n_bit >= 1 && n_bit <= 7, "uint8 norm codes need n_bit 1..7 (got %d)", n_bit);
+    GQ_REQUIRE(accumulate >= 0 && accumulate <= 2, "accumulate must be 0, 1 or 2");
+    GQ_REQUIRE(codes && l && lbub && u && minmax_keys, "null pointer");
+    GQ_REQUIRE((((uintptr_t)codes | (uintptr_t)l | (uintptr_t)lbub | (uintptr_t)u | (uintptr_t)uniforms |
+                 (uintptr_t)out) & 15) == 0,
+               "codes, l, lbub, u, uniforms and out must be 16-byte aligned");
+    set_rider(pending);
+    e = hsq_decode_quantize(codes, l, lbub, u, minmax_keys, n_chunks, codebook, seg_start, n_seg, n_bit, random,
+                            uniforms, philox_seed, philox_offset, accumulate, out, as_stream(stream));
+    const Rider left = take_rider();
+    if (e) return e;
+    return launch_rider(left, as_stream(stream));   // no-op: the decode kernel carried it
+}
+
 int gq_hsq_decode_reduce(const void *codes, int code_bytes, const void *l, int l_bytes,
                          const float *lbub, const float *norms_f32, int64_t user_stride_bytes,
                          int n_users, int64_t n_chunks, int d, const float *codebook, int K,

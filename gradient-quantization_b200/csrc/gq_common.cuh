@@ -114,6 +114,23 @@ __device__ __forceinline__ float philox_uniform(uint64_t seed, uint64_t offset, 
     uint32_t x = (s == 0) ? w.x : (s == 1) ? w.y : (s == 2) ? w.z : w.w;
     return u01(x);
 }
+// the uniforms of logical indices i .. i + 3 (== philox_uniform of each): one Philox block when
+// offset + i is a multiple of 4, else the two blocks the four words straddle
+__device__ __forceinline__ void philox_uniform4(uint64_t seed, uint64_t offset, uint64_t i, float (&r)[4])
+{
+    const uint64_t g = offset + i;
+    const uint4 a = philox4x32_10(seed, g >> 2);
+    const uint32_t sh = (uint32_t)(g & 3u);
+    if (sh == 0) {
+        r[0] = u01(a.x); r[1] = u01(a.y); r[2] = u01(a.z); r[3] = u01(a.w);
+        return;
+    }
+    const uint4 b = philox4x32_10(seed, (g >> 2) + 1);
+    r[0] = u01(sh == 1 ? a.y : sh == 2 ? a.z : a.w);
+    r[1] = u01(sh == 1 ? a.z : sh == 2 ? a.w : b.x);
+    r[2] = u01(sh == 1 ? a.w : sh == 2 ? b.x : b.y);
+    r[3] = u01(sh == 1 ? b.x : sh == 2 ? b.y : b.z);
+}
 
 // --------------------------------------------------------- segment lookup ---
 // seg_start is sorted, seg_start[0] == 0, seg_start[n_seg] == n.  Returns s with
@@ -182,6 +199,50 @@ __device__ __forceinline__ int psc_level(float v, float lb, float ub, float s, i
         li += (prob > r) ? 1 : 0;
     }
     return li;
+}
+// psc_level() for lb != ub, with den = ub - lb computed by the caller (same operations)
+__device__ __forceinline__ int psc_level_nz(float v, float lb, float den, float s, int random, float r)
+{
+    const float scaled = fabsf(__fdiv_rn(__fsub_rn(v, lb), den)) * s;
+    const float c = fminf(fmaxf(scaled, 0.0f), s - 1.0f);
+    int li = (int)c;
+    if (random) li += (__fsub_rn(scaled, (float)li) > r) ? 1 : 0;
+    return li;
+}
+// Levels of the four consecutive chunks i0 .. i0 + 3 (i0 < n) from a tensor-boundary table and the
+// (lb, ub) pairs in shared memory.  `seg` is a tensor at or before i0's and is advanced to it.  When all
+// four chunks lie in one tensor (almost always) lb, ub and ub - lb are fetched once.  Every kernel that
+// quantizes norms in groups of four (the tcgen05 encode's tail, the stand-alone quantizer, the fused
+// quantize-and-decode) computes its levels here, so their records agree bit for bit.
+template <typename SegT, typename IdxT>
+__device__ __forceinline__ void psc_levels4(const float (&x)[4], const float (&r)[4], IdxT i0, IdxT n,
+                                            const SegT *s_seg, const float2 *s_lbub, int &seg, float s, int random,
+                                            int (&lv)[4])
+{
+    while (i0 >= s_seg[seg + 1]) ++seg;
+    if (i0 + 3 < s_seg[seg + 1]) {
+        const float2 b = s_lbub[seg];
+        if (b.x - b.y == 0.0f) {
+            lv[0] = lv[1] = lv[2] = lv[3] = 0;
+        } else {
+            const float den = __fsub_rn(b.y, b.x);
+#pragma unroll
+            for (int t = 0; t < 4; ++t) lv[t] = psc_level_nz(x[t], b.x, den, s, random, r[t]);
+        }
+    } else {
+        int sg = seg;
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+            const IdxT i = i0 + t;
+            if (i < n) {
+                while (i >= s_seg[sg + 1]) ++sg;
+                const float2 b = s_lbub[sg];
+                lv[t] = psc_level(x[t], b.x, b.y, s, random, r[t]);
+            } else {
+                lv[t] = 0;
+            }
+        }
+    }
 }
 // ProbabilisticScalarCompressor.decompress (probabilistic_scalar_compressor.py:31-32)
 // s = 2^n is a power of two, so "/ s" is done as an exact multiplication by inv_s = 1/s

@@ -154,6 +154,12 @@ int hsq_decode_reduce(const void *codes, int code_bytes, const void *l, int l_by
                       int64_t n_chunks, int d,
                       const float *codebook, int K, const int64_t *seg_start, int n_seg, int n_bit,
                       int mean, int accumulate, float *out, cudaStream_t st);
+// one user's record whose levels the decode computes itself (d = 16, K = 256, uint8 codes and levels):
+// the norm quantization of the search that left u and the min/max keys behind, then the decode
+int hsq_decode_quantize(const void *codes, void *l, float *lbub, const float *u, const uint32_t *keys,
+                        int64_t n_chunks, const float *codebook, const int64_t *seg_start, int n_seg, int n_bit,
+                        int random, const float *uniforms, uint64_t seed, uint64_t offset, int accumulate,
+                        float *out, cudaStream_t st);
 int launch_f32_reduce_users(const float *in, int64_t user_stride, const int64_t *user_offsets, int n_users,
                             int64_t n, int mean, int accumulate, float *out, cudaStream_t st);
 int launch_axpy(const float *a, const float *b, float alpha, int64_t n, float *out, int sub,

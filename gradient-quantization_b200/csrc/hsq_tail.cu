@@ -9,6 +9,8 @@
 //   quantize: (4 u + 1 l [+4 r]) / d        decode-reduce: 4 + 2U/d (+4 if accumulate)
 #include <stdlib.h>
 
+#include <type_traits>
+
 #include "gq_internal.cuh"
 
 namespace gq {
@@ -70,15 +72,6 @@ norm_quantize_kernel(const float *__restrict__ u, int64_t n, const int64_t *__re
 // of one item each were 1.2 waves on 148 SMs: the second, nearly empty wave doubled the run
 // time); the loads of the next item are issued before the current one is processed.
 constexpr int kQuantMaxSeg = 1024;
-__device__ __forceinline__ int psc_level_nz(float v, float lb, float den, float s, int random, float r)
-{
-    // psc_level() for lb != ub, with den = ub - lb computed by the caller (same operations)
-    const float scaled = fabsf(__fdiv_rn(__fsub_rn(v, lb), den)) * s;
-    const float c = fminf(fmaxf(scaled, 0.0f), s - 1.0f);
-    int li = (int)c;
-    if (random) li += (__fsub_rn(scaled, (float)li) > r) ? 1 : 0;
-    return li;
-}
 template <typename LT>
 __global__ void __launch_bounds__(256)
 norm_quantize_smem_kernel(const float *__restrict__ u, int n, const int64_t *__restrict__ seg_start,
@@ -145,30 +138,8 @@ norm_quantize_smem_kernel(const float *__restrict__ u, int n, const int64_t *__r
             }
         }
         int seg = base < 0 ? 0 : base;
-        while (i0 >= s_segi[seg + 1]) ++seg;
         int lv[4];
-        if (i0 + 3 < s_segi[seg + 1]) {   // all four chunks in one tensor
-            const float2 b = s_lbub2[seg];
-            if (b.x - b.y == 0.0f) {
-                lv[0] = lv[1] = lv[2] = lv[3] = 0;
-            } else {
-                const float den = __fsub_rn(b.y, b.x);
-#pragma unroll
-                for (int t = 0; t < 4; ++t) lv[t] = psc_level_nz(x[t], b.x, den, s, random, r[t]);
-            }
-        } else {
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                const int i = i0 + t;
-                if (i < n) {
-                    while (i >= s_segi[seg + 1]) ++seg;
-                    const float2 b = s_lbub2[seg];
-                    lv[t] = psc_level(x[t], b.x, b.y, s, random, r[t]);
-                } else {
-                    lv[t] = 0;
-                }
-            }
-        }
+        psc_levels4(x, r, i0, n, s_segi, s_lbub2, seg, s, random, lv);
         if (full) {
             if (sizeof(LT) == 1) {
                 reinterpret_cast<uint32_t *>(l)[q] =
@@ -573,6 +544,12 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc)
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)),
                  "l"(gsrc) : "memory");
 }
+// the first src_bytes (1..16) of the 16 come from gsrc, the rest is zero-filled
+__device__ __forceinline__ void cp_async16_part(void *smem_dst, const void *gsrc, int src_bytes)
+{
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)),
+                 "l"(gsrc), "r"(src_bytes) : "memory");
+}
 __device__ __forceinline__ float4 lds128(uint32_t saddr)
 {
     float4 r;
@@ -585,19 +562,37 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t saddr)
     asm volatile("ld.shared.u8 %0, [%1];" : "=r"(r) : "r"(saddr) : "memory");
     return r;
 }
+// QUANT (NU == 1): the record's levels are not there yet.  The search kernel left u and the per-tensor
+// min/max keys behind (gq_hsq_encode_search); this kernel builds lb/ub from the keys, stages each tile's
+// u in place of its level bytes, computes the tile's levels before decoding it (psc_levels4, as the
+// encode's tail does), stores them over the first quarter of the staged u and into the record, and
+// CTA 0 writes the lb/ub table: the record ends up complete.  The stage buffer grows from 2 KB to 5 KB,
+// which keeps five CTAs per SM within the shared memory (and 48 registers) of the plain NU = 1 decode.
+struct DecQuant {
+    const float *u;
+    const uint32_t *keys;
+    const float *uniforms;   // nullptr: Philox4x32-10 (seed, offset + chunk)
+    uint64_t seed, offset;
+    int random;
+};
 // NU = exact number of users (compile time: the per-user loops are branch-free)
-template <int NU>
-__global__ void __launch_bounds__(kDecodeThreads)
-hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, const uint8_t *__restrict__ l,
-                                const float *__restrict__ lbub, const UserOffsets uoff,
+template <int NU, bool QUANT>
+__global__ void __launch_bounds__(kDecodeThreads, QUANT ? 5 : 0)
+hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__restrict__ l,
+                                float *__restrict__ lbub, const UserOffsets uoff,
                                 int64_t n_chunks, const float *__restrict__ codebook,
                                 const int64_t *__restrict__ seg_start, int n_seg, float s, int mean,
-                                int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait)
+                                int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait,
+                                const DecQuant quant)
 {
+    static_assert(!QUANT || NU == 1, "levels are computed for one user's record");
+    // one stage buffer: per user codes [1024] | levels [1024]; QUANT: codes [1024] | u [1024] (fp32), the
+    // levels overwrite the first 1024 bytes of u
+    constexpr int kBuf = NU * 2 * kStTile + (QUANT ? 3 * kStTile : 0);
     extern __shared__ float4 s_dyn[];
     float4 *s_cb = s_dyn;                                                    // [256][2][4]
-    uint8_t *s_stage = reinterpret_cast<uint8_t *>(s_cb + 256 * 8);          // [2][NU][codes 1024 | l 1024]
-    float2 *s_lbub = reinterpret_cast<float2 *>(s_stage + 2 * NU * 2 * kStTile);   // [NU][n_seg]
+    uint8_t *s_stage = reinterpret_cast<uint8_t *>(s_cb + 256 * 8);          // [2][kBuf]
+    float2 *s_lbub = reinterpret_cast<float2 *>(s_stage + 2 * kBuf);         // [NU][n_seg]
     int64_t *s_seg = reinterpret_cast<int64_t *>(s_lbub + NU * n_seg);             // [n_seg + 1] tensor boundaries
     __shared__ int64_t s_off[8];
     const int tid = threadIdx.x, lane = tid & 31;
@@ -622,13 +617,28 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, const uint8_t
     auto issue = [&](int64_t tile, int buf) {
         const int64_t c0 = tile * kStTile;
         const int64_t left = n_chunks - c0;
-        const int pieces = (int)(((left < kStTile ? left : (int64_t)kStTile) + 15) >> 4);   // 16-byte pieces holding data
+        const int lim = (int)(left < kStTile ? left : (int64_t)kStTile);
+        const int pieces = (lim + 15) >> 4;   // 16-byte pieces holding data
+        if (QUANT) {   // codes, then u: 64 + 256 pieces
+            for (int i = tid; i < 64 + 256; i += kDecodeThreads) {
+                if (i < 64) {
+                    if (i < pieces) cp_async16(s_stage + buf * kBuf + i * 16, codes + c0 + i * 16);
+                } else {
+                    const int p = i - 64;   // chunks 4p .. 4p + 3 of the tile
+                    if (4 * p < lim)
+                        cp_async16_part(s_stage + buf * kBuf + kStTile + p * 16, quant.u + c0 + 4 * p,
+                                        4 * min(4, lim - 4 * p));
+                }
+            }
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            return;
+        }
         for (int i = tid; i < NU * 128; i += kDecodeThreads) {
             const int u = i >> 7, which = (i >> 6) & 1, piece = i & 63;
             if (piece < pieces) {
                 const char *src = (which ? reinterpret_cast<const char *>(l) : reinterpret_cast<const char *>(codes)) +
                                   s_off[u] + c0 + piece * 16;
-                cp_async16(s_stage + ((buf * NU + u) * 2 + which) * kStTile + piece * 16, src);
+                cp_async16(s_stage + buf * kBuf + (u * 2 + which) * kStTile + piece * 16, src);
             }
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
@@ -643,20 +653,32 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, const uint8_t
     SegCache segc;
     float4 *o4 = reinterpret_cast<float4 *>(out);
     const int64_t n4 = n_chunks * 4;
-    int64_t tile = blockIdx.x;
+    // (32-bit tile indices in the QUANT kernel: what keeps it within 48 registers without spills)
+    std::conditional_t<QUANT, int, int64_t> tile = blockIdx.x;
     int buf = 0;
     if (tile < n_tiles) issue(tile, 0);
     // while the first tile is in flight: the users' (lb, ub) tables (read before the first decode,
     // i.e. after the block barrier that follows the tile's arrival) ...
-    for (int i = tid; i < NU * n_seg; i += kDecodeThreads) {
-        const int u = i / n_seg, sg = i - u * n_seg;
-        const float2 *b = reinterpret_cast<const float2 *>(reinterpret_cast<const char *>(lbub) + s_off[u]);
-        s_lbub[i] = __ldcv(b + sg);
+    if (QUANT) {
+        for (int i = tid; i < n_seg; i += kDecodeThreads) {
+            const float lb = key_to_float(__ldcg(quant.keys + 2 * i)), ub = key_to_float(__ldcg(quant.keys + 2 * i + 1));
+            s_lbub[i] = make_float2(lb, ub);
+            if (blockIdx.x == 0) {   // the reference returns lb/ub (probabilistic_scalar_compressor.py:27)
+                lbub[2 * i] = lb;
+                lbub[2 * i + 1] = ub;
+            }
+        }
+    } else {
+        for (int i = tid; i < NU * n_seg; i += kDecodeThreads) {
+            const int u = i / n_seg, sg = i - u * n_seg;
+            const float2 *b = reinterpret_cast<const float2 *>(reinterpret_cast<const char *>(lbub) + s_off[u]);
+            s_lbub[i] = __ldcv(b + sg);
+        }
     }
     // ... and the attached small reduction (identity tensors)
     rider_run(rider, (int64_t)blockIdx.x * kDecodeThreads + tid, (int64_t)gridDim.x * kDecodeThreads);
     for (; tile < n_tiles; tile += gridDim.x, buf ^= 1) {
-        const int64_t next = tile + gridDim.x;
+        const auto next = tile + gridDim.x;
         if (next < n_tiles) {
             issue(next, buf ^ 1);
             asm volatile("cp.async.wait_group 1;" ::: "memory");
@@ -664,8 +686,47 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, const uint8_t
             asm volatile("cp.async.wait_group 0;" ::: "memory");
         }
         __syncthreads();
-        const uint32_t st = stage0 + (uint32_t)(buf * NU * 2 * kStTile);
+        const uint32_t st = stage0 + (uint32_t)(buf * kBuf);
         const int64_t c0 = tile * kStTile;
+        if (QUANT) {
+            // levels of chunks c0 + 4 tid .. + 3: into the record and, once every thread has read its u,
+            // over the first 1024 bytes of the staged u, where the decode below reads the level bytes
+            const int i0 = (int)c0 + 4 * tid, n = (int)n_chunks;   // n_chunks < 2^31 (gq_hsq_decode_quantize)
+            uint32_t packed = 0u;
+            uint32_t *s_lv = reinterpret_cast<uint32_t *>(s_stage + buf * kBuf + kStTile);
+            if (i0 < n) {
+                const float4 xv = reinterpret_cast<const float4 *>(s_lv)[tid];
+                const float x[4] = {xv.x, xv.y, xv.z, xv.w};
+                float r[4] = {0.f, 0.f, 0.f, 0.f};
+                if (quant.random) {
+                    if (quant.uniforms != nullptr) {
+                        if (i0 + 3 < n) {
+                            const float4 t = __ldg(reinterpret_cast<const float4 *>(quant.uniforms + i0));
+                            r[0] = t.x; r[1] = t.y; r[2] = t.z; r[3] = t.w;
+                        } else {
+#pragma unroll
+                            for (int t = 0; t < 4; ++t) r[t] = (i0 + t < n) ? __ldg(quant.uniforms + i0 + t) : 0.0f;
+                        }
+                    } else {
+                        philox_uniform4(quant.seed, quant.offset, (uint64_t)i0, r);
+                    }
+                }
+                int seg = cached_segment_smem(segc, s_seg, n_seg, (int64_t)i0);
+                int lv[4];
+                psc_levels4(x, r, i0, n, s_seg, s_lbub, seg, s, quant.random, lv);
+                packed = (uint32_t)lv[0] | ((uint32_t)lv[1] << 8) | ((uint32_t)lv[2] << 16) | ((uint32_t)lv[3] << 24);
+                if (i0 + 3 < n) {
+                    reinterpret_cast<uint32_t *>(l)[i0 >> 2] = packed;
+                } else {
+#pragma unroll
+                    for (int t = 0; t < 4; ++t)
+                        if (i0 + t < n) l[i0 + t] = (uint8_t)lv[t];
+                }
+            }
+            __syncthreads();
+            s_lv[tid] = packed;
+            __syncthreads();
+        }
         for (int sl = warp; sl < kStTile / 32; sl += kDecodeThreads / 32) {
             const int64_t c = c0 + sl * 32 + lane;
             if (c0 + sl * 32 >= n_chunks) break;
@@ -759,13 +820,15 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, const uint8_t
     }
 }
 
-template <int NU>
+template <int NU, bool QUANT = false>
 static int launch_decode_staged(const void *codes, const void *l, const float *lbub, const UserOffsets &uoff,
                                 int64_t n_chunks, const float *codebook, const int64_t *seg_start,
-                                int n_seg, float s, int mean, int accumulate, float *out, cudaStream_t st)
+                                int n_seg, float s, int mean, int accumulate, float *out, cudaStream_t st,
+                                const DecQuant &quant = DecQuant{})
 {
-    auto kern = hsq_decode_reduce_staged_kernel<NU>;
-    const size_t smem = 256 * 128 + (size_t)2 * NU * 2 * kStTile + (size_t)NU * n_seg * 8 + (size_t)(n_seg + 1) * 8;
+    auto kern = hsq_decode_reduce_staged_kernel<NU, QUANT>;
+    const size_t buf = (size_t)NU * 2 * kStTile + (QUANT ? 3 * kStTile : 0);
+    const size_t smem = 256 * 128 + 2 * buf + (size_t)NU * n_seg * 8 + (size_t)(n_seg + 1) * 8;
     GQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 1;
     GQ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kDecodeThreads, smem));
@@ -778,9 +841,20 @@ static int launch_decode_staged(const void *codes, const void *l, const float *l
     const Rider rider = take_rider();   // carried by this launch if one is pending
     const PeerWait wait = take_wait();  // likewise: the wait for the peers' delivery flags
     GQ_CUDA(launch_pdl(kern, dim3((unsigned)grid), dim3(kDecodeThreads), smem, st, (const uint8_t *)codes,
-                       (const uint8_t *)l, lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean,
-                       accumulate, out, rider, wait));
+                       (uint8_t *)l, (float *)lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean,
+                       accumulate, out, rider, wait, quant));
     return GQ_OK;
+}
+
+int hsq_decode_quantize(const void *codes, void *l, float *lbub, const float *u, const uint32_t *keys,
+                        int64_t n_chunks, const float *codebook, const int64_t *seg_start, int n_seg, int n_bit,
+                        int random, const float *uniforms, uint64_t seed, uint64_t offset, int accumulate,
+                        float *out, cudaStream_t st)
+{
+    UserOffsets uoff = {};
+    const DecQuant quant = {u, keys, uniforms, seed, offset, random};
+    return launch_decode_staged<1, true>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg,
+                                         (float)(1u << n_bit), 0, accumulate, out, st, quant);
 }
 
 template <int D, int MAXU, typename CodeT, typename LT>

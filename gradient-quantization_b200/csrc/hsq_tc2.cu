@@ -841,37 +841,8 @@ hsq_encode_tc2_kernel(const __grid_constant__ CUtensorMap map_grad, const __grid
             const int i0 = q * 4;
             const float x[4] = {xv[j].x, xv[j].y, xv[j].z, xv[j].w};
             const float r[4] = {rv[j].x, rv[j].y, rv[j].z, rv[j].w};
-            while (i0 >= s_seg[seg + 1]) ++seg;
             int lv[4];
-            if (i0 + 3 < s_seg[seg + 1]) {   // all four chunks in one tensor
-                const float2 bb = s_lbub[seg];
-                if (bb.x - bb.y == 0.0f) {
-                    lv[0] = lv[1] = lv[2] = lv[3] = 0;
-                } else {
-                    const float den = __fsub_rn(bb.y, bb.x);
-#pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const float scaled = fabsf(__fdiv_rn(__fsub_rn(x[t], bb.x), den)) * s;
-                        const float cl = fminf(fmaxf(scaled, 0.0f), s - 1.0f);
-                        int li = (int)cl;
-                        if (random) li += (__fsub_rn(scaled, (float)li) > r[t]) ? 1 : 0;
-                        lv[t] = li;
-                    }
-                }
-            } else {
-                int sg = seg;
-#pragma unroll
-                for (int t = 0; t < 4; ++t) {
-                    const int i = i0 + t;
-                    if (i < n_chunks) {
-                        while (i >= s_seg[sg + 1]) ++sg;
-                        const float2 bb = s_lbub[sg];
-                        lv[t] = psc_level(x[t], bb.x, bb.y, s, random, r[t]);
-                    } else {
-                        lv[t] = 0;
-                    }
-                }
-            }
+            psc_levels4(x, r, i0, n_chunks, s_seg, s_lbub, seg, s, random, lv);
             packed = (uint32_t)lv[0] | ((uint32_t)lv[1] << 8) | ((uint32_t)lv[2] << 16) | ((uint32_t)lv[3] << 24);
             if (i0 + 3 < n_chunks) {
                 reinterpret_cast<uint32_t *>(P.l)[q] = packed;

@@ -17,6 +17,8 @@ NCCL all-gather with one user per rank -- and decode is one fused
 decode-and-reduce launch per group over all U records, in user order.
 Every section starts on a 256-byte boundary.
 """
+import os
+
 import torch
 
 from .. import _lib
@@ -68,9 +70,22 @@ class FusedPlan:
         self._classify()
         self._layout()
         self.arena = torch.zeros(self.arena_elems, dtype=torch.float32, device=device)
-        self.records = torch.zeros(n_users, self.record_bytes, dtype=torch.uint8, device=device)
+        self._records = torch.zeros(n_users, self.record_bytes, dtype=torch.uint8, device=device)
+        self._pending = None   # deferred levels: (row, group, seed, offset, uniforms) of the last encode
         self.workspace = torch.empty(max(self.workspace_bytes, _ALIGN), dtype=torch.uint8, device=device)
         self.u_scratch = torch.empty(max(self.max_chunks, 1), dtype=torch.float32, device=device)
+
+    @property
+    def records(self):
+        """[rows, record_bytes] uint8: the packed records.  Reading it completes a record whose levels
+        an encode(defer_levels=True) left to the next decode."""
+        self._complete()
+        return self._records
+
+    @records.setter
+    def records(self, buf):
+        self._complete()
+        self._records = buf
 
     # ------------------------------------------------------------ planning ---
     def _classify(self):
@@ -369,10 +384,15 @@ class FusedPlan:
         return out, pos
 
     # --------------------------------------------------------------- encode ---
-    def encode(self, user, src=None, uniforms=None, rng_user=None, shared_rng=False, part=None):
+    def encode(self, user, src=None, uniforms=None, rng_user=None, shared_rng=False, part=None, defer_levels=False):
         """Compress the arena (or `src`, laid out like it) into records[user].
         rng_user: logical user whose Philox stream the stochastic rounding draws from (default: the
         record row); shared_rng: the rank-independent stream instead (second phase of --two-phase).
+        defer_levels: on a plan that can_defer_levels(), launch only the search and leave the norm
+        quantization to the next decode of this one record, which then computes the levels itself
+        (gq_hsq_decode_quantize): the encode loses its grid barrier and tail, the step one kernel
+        phase.  Any other use of the record -- reading `records`, another decode, an encode of another
+        row -- completes it first with the stand-alone quantizer.  The bytes are the same either way.
         Launches: HSQ 2 per group on the tcgen05 path (search, quantize; 3 with the separate init
         kernel of the exact path), QSGD 1 (chunked) or 3, sign 1, top-k 10; the copy of the identity tensors rides
         in the first HSQ group's first kernel (1 launch of its own when there is no HSQ group)."""
@@ -380,7 +400,12 @@ class FusedPlan:
         src_ptr = src if isinstance(src, int) else src.data_ptr()   # tensor or raw device address
         rng_user = user if rng_user is None else rng_user
         take = _lib.PHILOX.take_shared if shared_rng else (lambda n: _lib.PHILOX.take(n, rng_user))
-        rec = self.records[user]
+        if self._pending is not None:
+            if part is None and self._pending[0] == user:
+                self._pending = None        # codes, u and keys of that row are about to be overwritten
+            else:
+                self._complete()            # u_scratch and the keys are shared by every row
+        rec = self._records[user]
         st = _lib.stream()
         base = rec.data_ptr()
         ident, carrier = self._rider_pair()
@@ -418,7 +443,12 @@ class FusedPlan:
             if g.kind == "hsq":
                 n_rand = g.n_chunks if (self.random and g.n_bit != 32) else 0
                 seed, off = take(n_rand) if (n_rand and r is None) else (0, 0)
-                if g.n_bit == 32:
+                if defer_levels and part is None and self.can_defer_levels():
+                    _lib.call("gq_hsq_encode_search", gp, g.n_chunks, g.dim, _lib.ptr(g.codebook), g.K,
+                              _lib.ptr(g.seg_start), g.n_seg, base + g.codes_off, g.code_bytes,
+                              _lib.ptr(self.u_scratch), _lib.ptr(self.workspace), self.workspace.numel(), st)
+                    self._pending = (user, g, seed, off, r)
+                elif g.n_bit == 32:
                     _lib.call("gq_hsq_encode", gp, g.n_chunks, g.dim, _lib.ptr(g.codebook), g.K,
                               _lib.ptr(g.seg_start), g.n_seg, 32, 0, None, 0, 0, base + g.codes_off,
                               g.code_bytes, None, 4, None, base + g.l_off, _lib.ptr(self.workspace),
@@ -483,6 +513,34 @@ class FusedPlan:
         return (g.dim in (8, 16, 32) and g.K == 256 and g.code_bytes == 1 and g.n_bit <= 7 and g.l_bytes == 1
                 and g.n_seg <= 1024 and g.n_chunks > 0)
 
+    def can_defer_levels(self):
+        """encode(defer_levels=True) defers the norm quantization on this plan: a single HSQ group of the
+        headline shape on the second-generation tcgen05 path (d = 16, K = 256, uint8 codes and levels,
+        n_bit <= 7, at most 1024 tensors), not cut into ring parts.  GQ_DEFER_LEVELS=0 turns it off
+        (read at every call, so one process can A/B the two)."""
+        if os.environ.get("GQ_DEFER_LEVELS", "1") == "0":
+            return False
+        if os.environ.get("GQ_TC_V", "2") == "1" or self.algo == _lib.ALGO_EXACT:
+            return False
+        hsq = [g for g in self.groups if g.kind != "identity"]
+        if len(hsq) != 1 or hsq[0].kind != "hsq":
+            return False
+        g = hsq[0]
+        return (g.dim == 16 and g.K == 256 and g.code_bytes == 1 and g.l_bytes == 1 and 1 <= g.n_bit <= 7
+                and g.n_seg <= 1024 and g.n_chunks > 0 and getattr(g, "part_cuts", None) is None)
+
+    def _complete(self):
+        """Write the levels and lb/ub of the record an encode(defer_levels=True) left pending (one
+        launch of the stand-alone quantizer over the search's u and min/max keys)."""
+        if self._pending is None:
+            return
+        row, g, seed, off, r = self._pending
+        self._pending = None
+        base = self._records.data_ptr() + row * self.record_bytes
+        _lib.call("gq_norm_quantize", _lib.ptr(self.u_scratch), g.n_chunks, _lib.ptr(g.seg_start), g.n_seg, g.n_bit,
+                  self.random, _lib.ptr(r), seed, off, base + g.l_off, g.l_bytes, base + g.lbub_off,
+                  _lib.ptr(self.workspace), 1, _lib.stream())
+
     def supports_inplace_feedback(self):
         """Error feedback without extra sweeps needs decode kernels with the subtract mode
         (accumulate = 2): everything but the top-k scatter."""
@@ -499,6 +557,11 @@ class FusedPlan:
         mean = 1 if mean else 0
         acc = int(accumulate)            # 0 store, 1 out += decoded, 2 out -= decoded (error feedback)
         ident, carrier = self._rider_pair(n_users)
+        pending = self._pending
+        if pending is not None and not (user_offsets is None and part is None and n_users == 1
+                                        and first_user == pending[0]):
+            self._complete()
+            pending = None
         if user_offsets is not None:
             for g in self.groups:
                 op = out.data_ptr() + g.arena_off * 4
@@ -514,7 +577,7 @@ class FusedPlan:
                     _lib.call("gq_f32_reduce_users_scattered", base_ptr + g.raw_off, user_offsets, n_users, g.n,
                               mean, acc, op, st)
             return out
-        base = self.records.data_ptr() + first_user * self.record_bytes
+        base = self._records.data_ptr() + first_user * self.record_bytes
         stride = self.record_bytes
         for g in self.groups:
             op = out.data_ptr() + g.arena_off * 4
@@ -538,7 +601,14 @@ class FusedPlan:
                 _lib.call("gq_attach_f32_reduce", base + ident.raw_off, stride, None, n_users, ident.n, mean, acc,
                           out.data_ptr() + ident.arena_off * 4)
             if g.kind == "hsq":
-                if g.n_bit == 32:
+                if pending is not None:
+                    _, _, seed, off, r = pending
+                    self._pending = None
+                    _lib.call("gq_hsq_decode_quantize", base + g.codes_off, base + g.l_off, base + g.lbub_off,
+                              _lib.ptr(self.u_scratch), _lib.ptr(self.workspace), g.n_chunks, g.dim,
+                              _lib.ptr(g.codebook), g.K, _lib.ptr(g.seg_start), g.n_seg, g.n_bit, self.random,
+                              _lib.ptr(r), seed, off, acc, op, st)
+                elif g.n_bit == 32:
                     _lib.call("gq_hsq_decode_reduce", base + g.codes_off, g.code_bytes, None, 1, None,
                               base + g.l_off, stride, n_users, g.n_chunks, g.dim, _lib.ptr(g.codebook), g.K,
                               _lib.ptr(g.seg_start), g.n_seg, 32, mean, acc, op, st)

@@ -142,10 +142,14 @@ class PSQuantizer(QuantizerBase):
 
     def _encode(self, slot, user, src=None, uniforms=None):
         """Fused encode of `user`'s gradient into row `slot`; with the fused peer-to-peer push the same
-        launch also delivers the record to every rank and announces the step epoch."""
+        launch also delivers the record to every rank and announces the step epoch.  With one user in
+        one process the record is decoded right after it is made (apply(), or the error feedback's
+        decode), so the norm quantization moves into that decode (FusedPlan.encode(defer_levels=True));
+        across processes the levels must exist before the record leaves the GPU."""
         if self.fused_push:
             self.p2p.attach_delivery(self.plan)
-        self.plan.encode(slot, src=src, uniforms=uniforms, rng_user=user)
+        defer = not self.distributed and self.plan.n_users == 1 and self.p2p is None
+        self.plan.encode(slot, src=src, uniforms=uniforms, rng_user=user, defer_levels=defer)
 
     def _scratch(self):
         if not hasattr(self, "_scratch_buf"):
@@ -239,7 +243,7 @@ class PSQuantizer(QuantizerBase):
                 for p, v in zip(self.parameters, self.plan.views(self._server_err)):
                     p.server_error = v
             p2.gather(self.plan.views(g), buf=self._server_err, feedback=1, scale=1.0)
-            p2.encode(0, src=self._server_err, uniforms=uniforms, shared_rng=True)
+            p2.encode(0, src=self._server_err, uniforms=uniforms, shared_rng=True, defer_levels=True)
             p2.decode(mean=False, out=g)
             p2.decode(mean=False, accumulate=2, out=self._server_err)
             return g
@@ -249,7 +253,7 @@ class PSQuantizer(QuantizerBase):
                 for p, v in zip(self.parameters, self.plan.views(self._server_err)):
                     p.server_error = v
             _lib.call("gq_axpy", _lib.ptr(g), _lib.ptr(self._server_err), 1.0, n, _lib.ptr(g), _lib.stream())
-        p2.encode(0, src=g, uniforms=uniforms, shared_rng=True)
+        p2.encode(0, src=g, uniforms=uniforms, shared_rng=True, defer_levels=True)
         dec = p2.decode(mean=False, out=self._scratch())
         if self.error_feedback:
             _lib.call("gq_sub", _lib.ptr(g), _lib.ptr(dec), n, _lib.ptr(self._server_err), _lib.stream())

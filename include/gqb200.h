@@ -141,6 +141,27 @@ int gq_hsq_decode_reduce(const void *codes, int code_bytes, const void *l, int l
  * equally spaced -- with peer-to-peer exchange each user's record lives in another GPU's memory
  * (mapped with gq_ipc_open) and is read over NVLink by the decode kernel itself.
  * Chunk dims 4, 8, 16 with a codebook of at most 64 KB; quantized norms only. */
+/* One user's encode and decode with the norm quantization moved from the encode into the decode
+ * (HSQ d = 16, K = 256, uint8 codes and levels, n_bit 1..7, n_seg <= 1024; tcgen05 search).  The
+ * quantization needs every tensor's final min/max, i.e. a grid-wide point after the search; the
+ * boundary between the two kernels provides it without a barrier inside the encode.
+ * gq_hsq_encode_search: gq_hsq_encode without the norm quantization -- writes codes and u_out and
+ *   leaves the per-tensor min/max keys in the workspace (its first 2*n_seg uint32 words); l and lbub
+ *   are not written.  Carries a pending gq_attach_f32_reduce like gq_hsq_encode.
+ * gq_hsq_decode_quantize: the rest of that encode fused into gq_hsq_decode_reduce with n_users = 1:
+ *   reads u and the keys (minmax_keys = that workspace), writes l and lbub into the record -- the same
+ *   bytes gq_hsq_encode writes for the same Philox range or uniforms -- and decodes the record into
+ *   out (accumulate 0, 1, 2 as in gq_hsq_decode_reduce).  Pointers 16-byte aligned.
+ * A record that must be complete without being decoded: gq_norm_quantize(u_out, ..., minmax_keys =
+ * the workspace, precomputed = 1) gives the same l and lbub. */
+int gq_hsq_encode_search(const float *grad, int64_t n_chunks, int d, const float *codebook, int K,
+                         const int64_t *seg_start, int n_seg, void *codes, int code_bytes, float *u_out,
+                         void *workspace, size_t workspace_bytes, gq_stream_t stream);
+int gq_hsq_decode_quantize(const void *codes, void *l, float *lbub, const float *u, const uint32_t *minmax_keys,
+                           int64_t n_chunks, int d, const float *codebook, int K, const int64_t *seg_start,
+                           int n_seg, int n_bit, int random, const float *uniforms, uint64_t philox_seed,
+                           uint64_t philox_offset, int accumulate, float *out, gq_stream_t stream);
+
 int gq_hsq_decode_reduce_scattered(const void *codes, int code_bytes, const void *l, int l_bytes,
                                    const float *lbub, const int64_t *user_byte_offsets, int n_users,
                                    int64_t n_chunks, int d, const float *codebook, int K,
