@@ -530,14 +530,18 @@ hsq_decode_reduce_warp_kernel(const CodeT *__restrict__ codes, const LT *__restr
 }
 
 // Pull-and-decode for records that live in DIFFERENT buffers (one per user, typically peer GPU
-// memory mapped over NVLink): d = 16, uint8 codes and levels.  Each CTA walks tiles of 1024 chunks;
-// the code / level bytes of all users for the next tile are pulled with 16-byte cp.async (wide
-// requests, bypassing L1) into a double-buffered shared-memory stage while the current tile is
-// decoded, so every remote byte crosses NVLink exactly once and the transfer overlaps the decode:
-// the exchange step needs no separate gather pass and no local copy of the peers' records.
-// The lb/ub tables of all users are staged once per CTA.  The codebook is stored twice per
-// codeword (128-byte slots): lanes 0-3 of a quarter-warp read the copy in bank groups 0-3, lanes
-// 4-7 the copy in groups 4-7, so the two codewords a quarter-warp gathers never conflict.
+// memory mapped over NVLink): d = 16 or 32, K = 256, uint8 codes and levels.  Each CTA walks tiles
+// of 1024 chunks; the code / level bytes of all users for the next tile are pulled with 16-byte
+// cp.async (wide requests, bypassing L1) into a double-buffered shared-memory stage while the
+// current tile is decoded, so every remote byte crosses NVLink exactly once and the transfer
+// overlaps the decode: the exchange step needs no separate gather pass and no local copy of the
+// peers' records.  The lb/ub tables of all users are staged once per CTA.  Every codeword has a
+// 128-byte slot in shared memory, and the D/4 lanes that write one chunk read their float4 from it
+// at (lane & 7) * 16:
+//   d = 16: the codeword is stored twice per slot: lanes 0-3 of a quarter-warp read the copy in bank
+//           groups 0-3, lanes 4-7 the copy in groups 4-7, so the two codewords a quarter-warp
+//           gathers never conflict;
+//   d = 32: the codeword fills the slot, and a quarter-warp reads exactly one codeword (all 32 banks).
 constexpr int kStTile = 1024;
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc)
 {
@@ -575,22 +579,25 @@ struct DecQuant {
     uint64_t seed, offset;
     int random;
 };
-// NU = exact number of users (compile time: the per-user loops are branch-free)
-template <int NU, bool QUANT>
-__global__ void __launch_bounds__(kDecodeThreads, QUANT ? 5 : 0)
-hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__restrict__ l,
-                                float *__restrict__ lbub, const UserOffsets uoff,
-                                int64_t n_chunks, const float *__restrict__ codebook,
-                                const int64_t *__restrict__ seg_start, int n_seg, float s, int mean,
-                                int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait,
-                                const DecQuant quant)
+// D = chunk dim (16 or 32), NU = exact number of users (compile time: the per-user loops are branch-free)
+template <int D, int NU, bool QUANT>
+__device__ __forceinline__ void
+hsq_decode_reduce_staged(const uint8_t *__restrict__ codes, uint8_t *__restrict__ l,
+                         float *__restrict__ lbub, const UserOffsets uoff,
+                         int64_t n_chunks, const float *__restrict__ codebook,
+                         const int64_t *__restrict__ seg_start, int n_seg, float s, int mean,
+                         int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait,
+                         const DecQuant quant)
 {
+    static_assert(D == 16 || D == 32, "staged decode: chunk dim 16 or 32");
     static_assert(!QUANT || NU == 1, "levels are computed for one user's record");
+    static_assert(!QUANT || D == 16, "deferred levels: d = 16 only");
+    constexpr int D4 = D / 4;   // float4 per chunk = lanes per chunk = rows of 32 float4 per warp slot
     // one stage buffer: per user codes [1024] | levels [1024]; QUANT: codes [1024] | u [1024] (fp32), the
     // levels overwrite the first 1024 bytes of u
     constexpr int kBuf = NU * 2 * kStTile + (QUANT ? 3 * kStTile : 0);
     extern __shared__ float4 s_dyn[];
-    float4 *s_cb = s_dyn;                                                    // [256][2][4]
+    float4 *s_cb = s_dyn;                                                    // [256][8]: d = 16 [2][4], d = 32 [8]
     uint8_t *s_stage = reinterpret_cast<uint8_t *>(s_cb + 256 * 8);          // [2][kBuf]
     float2 *s_lbub = reinterpret_cast<float2 *>(s_stage + 2 * kBuf);         // [NU][n_seg]
     int64_t *s_seg = reinterpret_cast<int64_t *>(s_lbub + NU * n_seg);             // [n_seg + 1] tensor boundaries
@@ -605,7 +612,7 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__re
         for (int u = 0; u < 8; ++u) s_off[u] = uoff.off[u];
     }
     for (int i = tid; i < 256 * 8; i += kDecodeThreads)
-        s_cb[i] = __ldg(reinterpret_cast<const float4 *>(codebook) + (i >> 3) * 4 + (i & 3));
+        s_cb[i] = __ldg(reinterpret_cast<const float4 *>(codebook) + (i >> 3) * D4 + (i & (D4 - 1)));
     for (int i = tid; i <= n_seg; i += kDecodeThreads) s_seg[i] = __ldg(seg_start + i);   // (a table of the plan, not of the step)
     __syncthreads();
     pdl_wait();   // the records are complete (and, across GPUs, announced by the barrier kernel)
@@ -648,11 +655,12 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__re
     constexpr bool pow2 = (NU & (NU - 1)) == 0;
     const float inv_nu = 1.0f / nu;
     // 32-bit shared-window addresses: this lane's 16-byte unit inside a codeword slot, the stage
+    // (the offset is (lane & 7) * 16; spelt as below, ptxas gives the d = 16 kernels 48 registers, not 53-57)
     const uint32_t cb_lane = (uint32_t)__cvta_generic_to_shared(s_cb) + (uint32_t)(((lane >> 2) & 1) * 64 + (lane & 3) * 16);
     const uint32_t stage0 = (uint32_t)__cvta_generic_to_shared(s_stage);
     SegCache segc;
     float4 *o4 = reinterpret_cast<float4 *>(out);
-    const int64_t n4 = n_chunks * 4;
+    const int64_t n4 = n_chunks * D4;
     // (32-bit tile indices in the QUANT kernel: what keeps it within 48 registers without spills)
     std::conditional_t<QUANT, int, int64_t> tile = blockIdx.x;
     int buf = 0;
@@ -759,10 +767,12 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__re
                     nrm[u] = __fadd_rn(__fmul_rn(__fmul_rn((float)(int)lv8, den[u]), inv_s), b.x);
                 }
             }
-            const int64_t f0 = (c0 + sl * 32) * 4;
+            // the slot's 32 * D4 float4 leave in D4 rows of 32 lanes (one contiguous 512-byte store each):
+            // float4 r * 32 + lane belongs to chunk r * (32 / D4) + lane / D4
+            const int64_t f0 = (c0 + sl * 32) * D4;
 #pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                const int owner = r * 8 + (lane >> 2);
+            for (int r = 0; r < D4; ++r) {
+                const int owner = r * (32 / D4) + lane / D4;
                 float4 cw[NU];
                 float nm[NU];
                 if (uni) {
@@ -820,13 +830,40 @@ hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__re
     }
 }
 
-template <int NU, bool QUANT = false>
+// one entry point per chunk dim (the d = 16 kernel keeps the name its profiles and tests know)
+template <int NU, bool QUANT>
+__global__ void __launch_bounds__(kDecodeThreads, QUANT ? 5 : 0)
+hsq_decode_reduce_staged_kernel(const uint8_t *__restrict__ codes, uint8_t *__restrict__ l,
+                                float *__restrict__ lbub, const UserOffsets uoff,
+                                int64_t n_chunks, const float *__restrict__ codebook,
+                                const int64_t *__restrict__ seg_start, int n_seg, float s, int mean,
+                                int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait,
+                                const DecQuant quant)
+{
+    hsq_decode_reduce_staged<16, NU, QUANT>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean,
+                                            accumulate, out, rider, wait, quant);
+}
+template <int NU>
+__global__ void __launch_bounds__(kDecodeThreads)
+hsq_decode_reduce_staged_d32_kernel(const uint8_t *__restrict__ codes, uint8_t *__restrict__ l,
+                                    float *__restrict__ lbub, const UserOffsets uoff,
+                                    int64_t n_chunks, const float *__restrict__ codebook,
+                                    const int64_t *__restrict__ seg_start, int n_seg, float s, int mean,
+                                    int accumulate, float *__restrict__ out, const Rider rider, const PeerWait wait,
+                                    const DecQuant quant)
+{
+    hsq_decode_reduce_staged<32, NU, false>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean,
+                                            accumulate, out, rider, wait, quant);
+}
+
+template <int D, int NU, bool QUANT = false>
 static int launch_decode_staged(const void *codes, const void *l, const float *lbub, const UserOffsets &uoff,
                                 int64_t n_chunks, const float *codebook, const int64_t *seg_start,
                                 int n_seg, float s, int mean, int accumulate, float *out, cudaStream_t st,
                                 const DecQuant &quant = DecQuant{})
 {
     auto kern = hsq_decode_reduce_staged_kernel<NU, QUANT>;
+    if constexpr (D == 32) kern = hsq_decode_reduce_staged_d32_kernel<NU>;
     const size_t buf = (size_t)NU * 2 * kStTile + (QUANT ? 3 * kStTile : 0);
     const size_t smem = 256 * 128 + 2 * buf + (size_t)NU * n_seg * 8 + (size_t)(n_seg + 1) * 8;
     GQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -853,8 +890,8 @@ int hsq_decode_quantize(const void *codes, void *l, float *lbub, const float *u,
 {
     UserOffsets uoff = {};
     const DecQuant quant = {u, keys, uniforms, seed, offset, random};
-    return launch_decode_staged<1, true>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg,
-                                         (float)(1u << n_bit), 0, accumulate, out, st, quant);
+    return launch_decode_staged<16, 1, true>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg,
+                                             (float)(1u << n_bit), 0, accumulate, out, st, quant);
 }
 
 template <int D, int MAXU, typename CodeT, typename LT>
@@ -891,21 +928,25 @@ static int launch_decode_d(const void *codes, const void *l, const float *lbub, 
     constexpr int D4c = D / 4;
     constexpr bool kWarpPath = ((D4c & (D4c - 1)) == 0) && D4c <= 4;   // D = 4, 8, 16
     constexpr int DW = kWarpPath ? D : 16;
-    if (kWarpPath && cb_bytes <= 64 * 1024 && n_users <= 8) {
-        UserOffsets uoff;
-        for (int u = 0; u < 8; ++u)
-            uoff.off[u] = (u < n_users) ? (user_offsets ? user_offsets[u] : (int64_t)u * user_stride) : 0;
+    UserOffsets uoff = {};
+    if (n_users <= 8) {
+        for (int u = 0; u < n_users; ++u)
+            uoff.off[u] = user_offsets ? user_offsets[u] : (int64_t)u * user_stride;
+    }
+    if constexpr (D == 16 || D == 32) {
         // records in separate (peer) buffers: pull-and-decode through a shared-memory stage
         // and for local records as well: measured faster than the warp kernel for every U
-        // (U = 1: 23 vs 27 us, U = 8: 76 vs 83 us on the ResNet-50 record); GQ_DECODE_STAGED=0 = old path
+        // (U = 1: 23 vs 27 us, U = 8: 76 vs 83 us on the ResNet-50 record; d = 32, B200 at 1000 W: U = 1
+        // 20.1 vs 33.1 us on the ResNet-50 gradient, 26.1-27.1 vs 26.8 us on the flat 25.6 M one, U = 8
+        // 48.4 vs 101.4 / 44.9 vs 98.0 us); GQ_DECODE_STAGED=0 = old path
         bool staged = true;
         if (const char *e = getenv("GQ_DECODE_STAGED")) staged = atoi(e) != 0;
-        if (staged && D == 16 && K == 256 && sizeof(CodeT) == 1 && sizeof(LT) == 1 && n_bit != 32 &&
+        if (staged && n_users <= 8 && K == 256 && sizeof(CodeT) == 1 && sizeof(LT) == 1 && n_bit != 32 &&
             (size_t)n_users * n_seg * 8 <= 48 * 1024) {
             bool aligned = (((uintptr_t)codes | (uintptr_t)l | (uintptr_t)lbub) & 15) == 0;
             for (int u = 0; u < n_users; ++u) aligned = aligned && ((uoff.off[u] & 15) == 0);
             if (aligned) {
-#define GQ_S(MU) case MU: return launch_decode_staged<MU>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean, accumulate, out, st)
+#define GQ_S(MU) case MU: return launch_decode_staged<D, MU>(codes, l, lbub, uoff, n_chunks, codebook, seg_start, n_seg, s, mean, accumulate, out, st)
                 switch (n_users) {
                     GQ_S(1); GQ_S(2); GQ_S(3); GQ_S(4); GQ_S(5); GQ_S(6); GQ_S(7); GQ_S(8);
                     default: break;
@@ -913,6 +954,8 @@ static int launch_decode_d(const void *codes, const void *l, const float *lbub, 
 #undef GQ_S
             }
         }
+    }
+    if (kWarpPath && cb_bytes <= 64 * 1024 && n_users <= 8) {
         GQ_CUDA_INT(flush_wait(st));
 #define GQ_W(MU) return launch_decode_warp<DW, MU, CodeT, LT>(codes, l, lbub, norms_f32, uoff, n_users, n_chunks, codebook, K, seg_start, n_seg, s, n_bit, mean, accumulate, out, st)
         if (n_users == 1) GQ_W(1);
@@ -922,7 +965,9 @@ static int launch_decode_d(const void *codes, const void *l, const float *lbub, 
 #undef GQ_W
     }
     if (user_offsets != nullptr) {
-        set_error("scattered user records need chunk dim 4/8/16, a codebook <= 64 KB and <= 8 users");
+        set_error("scattered user records need <= 8 users and chunk dim 4/8/16 with a codebook <= 64 KB, or chunk "
+                  "dim 32 with K = 256, uint8 codes and levels, n_users * n_seg <= 6144 and 16-byte aligned "
+                  "sections and user offsets");
         return GQ_ERR_UNSUPPORTED;
     }
     GQ_CUDA_INT(flush_wait(st));

@@ -491,18 +491,24 @@ class FusedPlan:
 
     # --------------------------------------------------------------- decode ---
     def supports_scattered(self):
-        """Peer-to-peer decode handles HSQ groups with chunk dim 4/8/16, a codebook of at most
-        64 KB and quantized norms, plus the identity tensors."""
+        """Peer-to-peer decode (gq_hsq_decode_reduce_scattered) handles quantized-norm HSQ groups with
+        chunk dim 4/8/16 and a codebook of at most 64 KB, or chunk dim 32 with K = 256, uint8 codes and
+        levels (n_bit <= 7) and the users' lb/ub tables within 48 KB, plus the identity tensors."""
         for g in self.groups:
             if g.kind == "identity":
                 continue
-            if g.kind != "hsq" or g.dim not in (4, 8, 16) or g.K * g.dim * 4 > 65536 or g.n_bit == 32:
+            if g.kind != "hsq" or g.n_bit == 32:
+                return False
+            if g.dim in (4, 8, 16) and g.K * g.dim * 4 <= 65536:
+                continue
+            if not (g.dim == 32 and g.K == 256 and g.code_bytes == 1 and g.l_bytes == 1
+                    and self.n_users * g.n_seg * 8 <= 48 * 1024):
                 return False
         return True
 
     def supports_fused_delivery(self):
         """The one-launch tcgen05 encode can deliver the record to the peers itself when the plan is a
-        single HSQ group of the headline shape (d = 16, K = 256, uint8 codes and levels) plus identity."""
+        single HSQ group with d = 8, 16 or 32, K = 256 and uint8 codes and levels, plus identity."""
         import os
         if os.environ.get("GQ_TC_V", "2") == "1" or self.algo == _lib.ALGO_EXACT:
             return False
@@ -656,7 +662,7 @@ class FusedPlan:
             n += (2 + n_users) if g.kind == "topk" else 1
         ident, carrier = self._rider_pair(n_users)
         if carrier is not None and (carrier.kind != "hsq" or (
-                carrier.dim == 16 and carrier.K == 256 and carrier.code_bytes == 1
+                carrier.dim in (16, 32) and carrier.K == 256 and carrier.code_bytes == 1
                 and carrier.l_bytes == 1 and carrier.n_bit != 32)):   # rides in the (staged) decode kernel
             n -= 1
         return n

@@ -46,7 +46,8 @@ class RingQuantizer(QuantizerBase):
         """Hops through peer-mapped memory: the encode kernel of rank r stores each stage of its record
         straight into rank r + 1's receive block and raises a flag the decode-accumulate kernel there
         waits on (the last rank: into every rank's block) -- the ps exchange's machinery, one target per
-        hop.  Needs the one-launch tcgen05 encode (HSQ d = 8 / 16, K = 256) on every rank."""
+        hop.  Needs the one-launch tcgen05 encode and the peer-to-peer decode (HSQ d = 8 / 16 / 32, K = 256,
+        FusedPlan.supports_fused_delivery and supports_scattered) on every rank."""
         import os
         import torch.distributed as dist
         want = getattr(self.args, "p2p", True) and os.environ.get("GQ_P2P", "1") != "0"

@@ -136,11 +136,6 @@ int gq_hsq_decode_reduce(const void *codes, int code_bytes, const void *l, int l
                          const int64_t *seg_start, int n_seg, int n_bit,
                          int mean, int accumulate, float *out, gq_stream_t stream);
 
-/* Same reduction, but user u's arrays are found at (pointer of user 0) + user_byte_offsets[u]
- * (host array, n_users <= 8, offsets may be any 64-bit distance): the packed records need not be
- * equally spaced -- with peer-to-peer exchange each user's record lives in another GPU's memory
- * (mapped with gq_ipc_open) and is read over NVLink by the decode kernel itself.
- * Chunk dims 4, 8, 16 with a codebook of at most 64 KB; quantized norms only. */
 /* One user's encode and decode with the norm quantization moved from the encode into the decode
  * (HSQ d = 16, K = 256, uint8 codes and levels, n_bit 1..7, n_seg <= 1024; tcgen05 search).  The
  * quantization needs every tensor's final min/max, i.e. a grid-wide point after the search; the
@@ -162,6 +157,16 @@ int gq_hsq_decode_quantize(const void *codes, void *l, float *lbub, const float 
                            int n_seg, int n_bit, int random, const float *uniforms, uint64_t philox_seed,
                            uint64_t philox_offset, int accumulate, float *out, gq_stream_t stream);
 
+/* Same reduction as gq_hsq_decode_reduce, but user u's arrays are found at (pointer of user 0) +
+ * user_byte_offsets[u] (host array, n_users <= 8, offsets may be any 64-bit distance): the packed
+ * records need not be equally spaced -- with peer-to-peer exchange each user's record lives in another
+ * GPU's memory (mapped with gq_ipc_open) and is read over NVLink by the decode kernel itself.
+ * Quantized norms only, and either
+ *   chunk dims 4, 8, 16 with a codebook of at most 64 KB, or
+ *   chunk dim 32 with K == 256, uint8 codes and levels (code_bytes == l_bytes == 1), the users' lb/ub
+ *   tables within 48 KB (n_users * n_seg <= 6144), and codes, l, lbub and every user offset 16-byte
+ *   aligned;
+ * anything else returns GQ_ERR_UNSUPPORTED. */
 int gq_hsq_decode_reduce_scattered(const void *codes, int code_bytes, const void *l, int l_bytes,
                                    const float *lbub, const int64_t *user_byte_offsets, int n_users,
                                    int64_t n_chunks, int d, const float *codebook, int K,
