@@ -54,6 +54,7 @@ _SIGNATURES = {
     "gq_peer_push": (c_int, [c_void_p, c_void_p, c_size, c_int, c_void_p]),
     "gq_peer_push_multicast": (c_int, [c_void_p, c_void_p, c_size, c_void_p]),
     "gq_attach_remote_record": (c_int, [c_int, c_int, c_void_p, c_void_p, c_i64, c_void_p, c_int, ctypes.c_uint32]),
+    "gq_attach_delivery_counter": (c_int, [c_void_p]),
     "gq_attach_peer_wait": (c_int, [c_void_p, c_int, ctypes.c_uint32]),
     "gq_f32_reduce_users": (c_int, [c_void_p, c_i64, c_int, c_i64, c_int, c_int, c_void_p, c_void_p]),
     "gq_qsgd_wire_bits": (c_int, [c_int]),

@@ -90,9 +90,49 @@ struct Tc2Remote {
     const uint8_t *ident;   // identity section inside the local record (mirrored too), may be null
     int64_t ident_bytes;
     uint32_t *flag[8];      // words that receive `epoch` (st.release.sys) when the record is delivered
+    int n_flag;             // 0: deliver, do not announce (an earlier launch of a multi-launch encode)
+    uint32_t epoch;
+    uint32_t *counter;      // arrival counter of the sign / QSGD encodes (gq_attach_delivery_counter)
+};
+// Where else the finished record sections go (multi-GPU exchange fused into the encode kernel):
+// every address a delivering kernel writes inside the local record is also written at address + delta[i].
+struct Remote {
+    int n;                  // number of remote destinations (0: none)
+    int multicast;          // 1: delta[0] leads into an NVLS multicast mapping (multimem.st)
+    int64_t delta[7];
+    const uint8_t *ident;   // identity section of the local record (written by the rider), mirrored too
+    int64_t ident_bytes;    // multiple of 16
+    uint32_t *done;         // arrival counter (HSQ: zeroed together with the grid barrier word; the
+                            // elementwise encodes: reset by the last CTA to arrive)
+    uint32_t *flag[8];      // where to announce `epoch` once every CTA has delivered (n_flag entries, may be 0)
     int n_flag;
     uint32_t epoch;
 };
+
+// store 4 bytes / 16 bytes at a local record address and at every remote copy of it
+__device__ __forceinline__ void remote_st32(const Remote &R, void *local, uint32_t v)
+{
+    if (R.multicast) {
+        asm volatile("multimem.st.weak.global.u32 [%0], %1;" ::"l"((char *)local + R.delta[0]), "r"(v) : "memory");
+    } else {
+#pragma unroll
+        for (int i = 0; i < 7; ++i)
+            if (i < R.n) *reinterpret_cast<uint32_t *>((char *)local + R.delta[i]) = v;
+    }
+}
+__device__ __forceinline__ void remote_st128(const Remote &R, void *local, uint4 v)
+{
+    if (R.multicast) {
+        asm volatile("multimem.st.weak.global.v4.f32 [%0], {%1, %2, %3, %4};"
+                     ::"l"((char *)local + R.delta[0]), "f"(__uint_as_float(v.x)), "f"(__uint_as_float(v.y)),
+                       "f"(__uint_as_float(v.z)), "f"(__uint_as_float(v.w)) : "memory");
+    } else {
+#pragma unroll
+        for (int i = 0; i < 7; ++i)
+            if (i < R.n) *reinterpret_cast<uint4 *>((char *)local + R.delta[i]) = v;
+    }
+}
+
 bool hsq_tc2_tail_supported(int n_seg, int n_bit, int l_bytes, const void *u_out, const void *uniforms, const void *l,
                             const void *codes);
 bool hsq_tc2_supported(int d, int K, int code_bytes);   // d in {8, 16, 32}, K == 256, uint8 codes

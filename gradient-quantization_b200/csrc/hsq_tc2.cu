@@ -79,20 +79,6 @@ struct Layout {
     static_assert(kStages * Dim<D>::kTileBytes >= 4 * (kTailMaxSeg + 2) + 8 * kTailMaxSeg, "tail tables live in the stage ring");
 };
 
-// Where else the finished record sections go (multi-GPU ps exchange fused into the encode):
-// every address the tail writes inside the local record is also written at address + delta[i].
-struct Remote {
-    int n;                  // number of remote destinations (0: none)
-    int multicast;          // 1: delta[0] leads into an NVLS multicast mapping (multimem.st)
-    int64_t delta[7];
-    const uint8_t *ident;   // identity section of the local record (written by the rider), mirrored too
-    int64_t ident_bytes;    // multiple of 16
-    uint32_t *done;         // local arrival counter (zeroed together with the grid barrier word)
-    uint32_t *flag[8];      // where to announce `epoch` once every CTA has delivered (n_flag entries)
-    int n_flag;
-    uint32_t epoch;
-};
-
 struct Enc2 {
     const float *codebook;
     int n_chunks;
@@ -162,30 +148,6 @@ __device__ __forceinline__ float pair_group_max(uint32_t pa, uint32_t ma, uint32
 {
     return fmaxf(__fadd_rn(fabsf(__uint_as_float(pa)), fabsf(__uint_as_float(ma))),
                  __fadd_rn(fabsf(__uint_as_float(pb)), fabsf(__uint_as_float(mb))));
-}
-
-// store 4 bytes / 16 bytes at a local record address and at every remote copy of it
-__device__ __forceinline__ void remote_st32(const Remote &R, void *local, uint32_t v)
-{
-    if (R.multicast) {
-        asm volatile("multimem.st.weak.global.u32 [%0], %1;" ::"l"((char *)local + R.delta[0]), "r"(v) : "memory");
-    } else {
-#pragma unroll
-        for (int i = 0; i < 7; ++i)
-            if (i < R.n) *reinterpret_cast<uint32_t *>((char *)local + R.delta[i]) = v;
-    }
-}
-__device__ __forceinline__ void remote_st128(const Remote &R, void *local, uint4 v)
-{
-    if (R.multicast) {
-        asm volatile("multimem.st.weak.global.v4.f32 [%0], {%1, %2, %3, %4};"
-                     ::"l"((char *)local + R.delta[0]), "f"(__uint_as_float(v.x)), "f"(__uint_as_float(v.y)),
-                       "f"(__uint_as_float(v.z)), "f"(__uint_as_float(v.w)) : "memory");
-    } else {
-#pragma unroll
-        for (int i = 0; i < 7; ++i)
-            if (i < R.n) *reinterpret_cast<uint4 *>((char *)local + R.delta[i]) = v;
-    }
 }
 
 // K-major operand descriptor: rows of one swizzle atom (32 / 64 / 128 B), 8-row groups 8 * row bytes apart

@@ -209,17 +209,22 @@ int gq_peer_push(const void *src, void *const *dst_ptrs, size_t bytes, int n_dst
     return GQ_OK;
 }
 
-// Fused exchange, sending side: the NEXT gq_hsq_encode on this host thread also stores every finished
-// section of the record it writes at (local address + delta[i]) for i < n_remote (peer-mapped copies of
-// the same record row), or once through an NVLS multicast mapping (multicast = 1, n_remote = 1), mirrors
-// the identity section [ident, ident + ident_bytes) the same way, and finally stores `epoch` into the
-// n_flags words flag_ptrs[i] (this rank's slot in every rank's flag array, its own included).
-// Requires the one-launch tcgen05 encode (d = 16, K = 256, uint8 codes and levels); otherwise that
-// encode fails with GQ_ERR_UNSUPPORTED and nothing is sent.
+// Fused exchange, sending side: the NEXT encode call on this host thread (gq_hsq_encode, gq_sign_encode,
+// gq_sign_encode_t5 or gq_qsgd_encode) also stores every finished section of the record it writes at
+// (local address + delta[i]) for i < n_remote (peer-mapped copies of the same record row), or once through
+// an NVLS multicast mapping (multicast = 1, n_remote = 1), mirrors the identity section
+// [ident, ident + ident_bytes) the same way, and finally stores `epoch` into the n_flags words flag_ptrs[i]
+// (this rank's slot in every rank's flag array, its own included).  n_flags == 0: deliver, do not announce
+// (every launch but the last of an encode made of several calls).
+// Requires a delivering kernel: the one-launch tcgen05 encode (d = 8, 16 or 32, K = 256, uint8 codes and
+// levels), the packed-words sign kernel, the base-3 sign kernel, the one-launch chunked QSGD kernel or the
+// TernGrad range kernels; the sign and QSGD ones also need gq_attach_delivery_counter.  Any other encode
+// fails with GQ_ERR_UNSUPPORTED and nothing is sent; the pending delivery is cleared either way.
 int gq_attach_remote_record(int n_remote, int multicast, const int64_t *delta, const void *ident, int64_t ident_bytes,
                             void *const *flag_ptrs, int n_flags, uint32_t epoch)
 {
-    GQ_REQUIRE(n_remote >= 1 && n_remote <= 7 && delta && flag_ptrs && n_flags >= 1 && n_flags <= 8, "bad arguments");
+    GQ_REQUIRE(n_remote >= 1 && n_remote <= 7 && delta && n_flags >= 0 && n_flags <= 8 && (flag_ptrs || n_flags == 0),
+               "bad arguments");
     GQ_REQUIRE(!multicast || n_remote == 1, "a multicast delivery has one destination");
     GQ_REQUIRE(ident_bytes >= 0 && ident_bytes % 16 == 0 && (ident_bytes == 0 || ((uintptr_t)ident & 15) == 0),
                "identity section must be 16-byte granular");
@@ -239,9 +244,23 @@ int gq_attach_remote_record(int n_remote, int multicast, const int64_t *delta, c
     return GQ_OK;
 }
 
-// Fused exchange, receiving side: the NEXT HSQ decode on this host thread first waits until all
-// n_ranks words of the local flag array have reached `epoch` (inside the decode kernel's prologue
-// when it is the staged kernel, else in a one-warp kernel launched before it).
+// The arrival counter of the pending delivery (after gq_attach_remote_record): a zero-initialised,
+// 4-byte aligned device word that no other delivery uses at the same time.  The sign and QSGD encodes
+// have no grid barrier behind which to zero one: their last CTA to arrive sets it back to 0.
+int gq_attach_delivery_counter(void *counter)
+{
+    Tc2Remote r = take_remote();
+    GQ_REQUIRE(r.n > 0, "no remote delivery is attached");
+    GQ_REQUIRE(counter && ((uintptr_t)counter & 3) == 0, "bad counter address");
+    r.counter = reinterpret_cast<uint32_t *>(counter);
+    set_remote(r);
+    return GQ_OK;
+}
+
+// Fused exchange, receiving side: the NEXT HSQ, sign or QSGD decode on this host thread first waits until
+// all n_ranks words of the local flag array have reached `epoch` (inside the decode kernel's prologue
+// when it is the staged HSQ kernel or a fast sign / QSGD kernel, else in a one-warp kernel launched
+// before it).
 int gq_attach_peer_wait(const void *local_flags, int n_ranks, uint32_t epoch)
 {
     GQ_REQUIRE(local_flags && n_ranks >= 1 && n_ranks <= 8, "bad arguments");

@@ -16,6 +16,95 @@ static int grid_for(int64_t n, int per_block, int waves = 8)
     return (int)(g < 1 ? 1 : g);
 }
 
+// ------------------------------------------------------ peer-to-peer delivery ---
+// The one-launch encodes below take `bool DELIVER` as a template parameter: with a remote delivery
+// attached (gq_attach_remote_record) they also store every record byte they write at the peers'
+// copies of the record, then run the arrival handshake; the DELIVER == false instantiations never
+// touch the Remote parameter and compile to the code of an encode without delivery.  These kernels
+// have no grid barrier, so
+//  - a section whose 32-bit words are written by different lanes or CTAs is sent by read-back: a
+//    CTA re-reads (ld.cg) what it wrote after a __syncthreads, and the words it shares with another
+//    CTA are sent by the last CTA to arrive, which sees every CTA's stores (deliver_finish);
+//  - the arrival counter cannot be zeroed in the prologue: the last CTA to arrive sets it back to 0.
+//    The next launch that counts on it runs its atomics after griddepcontrol.wait, i.e. after this
+//    grid has completed, reset included.
+
+// Remote copy of the local bytes [p0, p1) that this CTA has written and synchronised: whole 16-byte
+// words with one wide store, the 4-byte words before and after one by one.  A 32-bit word that the
+// range covers only in part is left to its neighbour's owner (deliver_finish).  Block-collective.
+__device__ __forceinline__ void deliver_bytes(const Remote &R, const void *p0, const void *p1)
+{
+    const uintptr_t a0 = ((uintptr_t)p0 + 3) & ~(uintptr_t)3, a1 = (uintptr_t)p1 & ~(uintptr_t)3;
+    if (a0 >= a1) return;
+    const uintptr_t v0 = min((a0 + 15) & ~(uintptr_t)15, a1), v1 = max(v0, a1 & ~(uintptr_t)15);
+    const uintptr_t t = threadIdx.x, nt = blockDim.x;
+    for (uintptr_t a = a0 + 4 * t; a < v0; a += 4 * nt) remote_st32(R, (void *)a, __ldcg((const uint32_t *)a));
+    for (uintptr_t a = v0 + 16 * t; a < v1; a += 16 * nt) remote_st128(R, (void *)a, __ldcg((const uint4 *)a));
+    for (uintptr_t a = v1 + 4 * t; a < a1; a += 4 * nt) remote_st32(R, (void *)a, __ldcg((const uint32_t *)a));
+}
+// the 32-bit word of the local record that holds byte p, read back and sent whole
+__device__ __forceinline__ void deliver_word(const Remote &R, const void *p)
+{
+    const uint32_t *w = reinterpret_cast<const uint32_t *>((uintptr_t)p & ~(uintptr_t)3);
+    remote_st32(R, const_cast<uint32_t *>(w), __ldcg(w));
+}
+
+// The identity section, when this launch carries it.  A rider of this launch wrote element i from grid
+// thread i (mod threads), the thread that reads it back here; one written by an earlier launch is
+// visible after griddepcontrol.wait.  Call after rider_run().
+__device__ __forceinline__ void deliver_ident(const Remote &R)
+{
+    const uint32_t *w = reinterpret_cast<const uint32_t *>(R.ident);
+    const int64_t nw = R.ident_bytes >> 2, nt = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nw; i += nt)
+        remote_st32(R, const_cast<uint32_t *>(w + i), __ldcg(w + i));
+}
+
+// End of a delivering launch, block-collective: every CTA makes its remote stores visible system-wide
+// and arrives on the counter; the last CTA to arrive runs last() (every CTA's local stores are visible
+// to it), sends what that wrote, sets the counter back to 0 and stores the epoch into the n_flag flag
+// words with st.release.sys (n_flag == 0: an earlier launch of a multi-launch encode, which delivers
+// and leaves the announcement to the last launch).
+template <typename F>
+__device__ __forceinline__ void deliver_finish(const Remote &R, F &&last)
+{
+    __shared__ int s_last;
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        s_last = atomicAdd(R.done, 1u) == gridDim.x - 1;
+        __threadfence();
+    }
+    __syncthreads();
+    if (!s_last) return;
+    last();
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) *R.done = 0u;
+    __syncthreads();
+    if ((int)threadIdx.x < R.n_flag)
+        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(R.flag[threadIdx.x]), "r"(R.epoch) : "memory");
+}
+
+// A PeerWait as a template-selected parameter of the fast decodes (WAIT == false: never touched).  With
+// WAIT every CTA polls the flags after griddepcontrol.wait and before it reads a record byte, and the
+// records are read with ld.global.cg instead of ld.global.nc: the peers write them while this grid is
+// resident, and the non-coherent path is only defined for data that is read-only for the kernel's life.
+template <bool WAIT>
+__device__ __forceinline__ void wait_prologue(const PeerWait &w)
+{
+    if constexpr (WAIT) {
+        if ((int)threadIdx.x < w.n) peer_wait_flag(w.flags + threadIdx.x, w.epoch, w.timeout_ns);
+        __syncthreads();
+    }
+}
+template <bool WAIT, typename T>
+__device__ __forceinline__ T ld_rec(const T *p)
+{
+    if constexpr (WAIT) return __ldcg(p);
+    else return __ldg(p);
+}
+
 __device__ __forceinline__ int64_t chunk_of(const int64_t *__restrict__ chunk_start, int64_t n_chunks,
                                             int dim, int64_t i)
 {
@@ -179,21 +268,25 @@ __device__ __forceinline__ void qsgd_uniforms4(int random, const float *__restri
     }
 }
 
-template <int BITS, int NV, int LPC, int UNR>
+template <int BITS, int NV, int LPC, int UNR, bool DELIVER>
 __global__ void __launch_bounds__(256)
 qsgd_encode_chunks_kernel(const float *__restrict__ v, int64_t n_chunks, int dim, float s, int random,
                           const float *__restrict__ uniforms, uint64_t seed, uint64_t offset,
-                          float *__restrict__ norm, void *__restrict__ packed, const Rider rider)
+                          float *__restrict__ norm, void *__restrict__ packed, const Rider rider, const Remote R)
 {
     pdl_launch_dependents();
     const int dim4 = dim >> 2;
     const int sub = threadIdx.x & (LPC - 1);
-    const int64_t n_slots = (int64_t)gridDim.x * (256 / LPC);
+    constexpr int SPB = 256 / LPC;   // chunk slots per CTA
+    const int64_t n_slots = (int64_t)gridDim.x * SPB;
     const int64_t slot = ((int64_t)blockIdx.x * 256 + threadIdx.x) / LPC;
     const int64_t warp_slot0 = (((int64_t)blockIdx.x * 256 + threadIdx.x) & ~31ll) / LPC;
+    // a delivering CTA ends every iteration with a __syncthreads: a CTA-uniform trip count
+    const int64_t first_slot = DELIVER ? (int64_t)blockIdx.x * SPB : warp_slot0;
     pdl_wait();
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
-    for (int64_t base = 0; base + warp_slot0 < n_chunks; base += n_slots * UNR) {   // warp-uniform trip count
+    if constexpr (DELIVER) deliver_ident(R);
+    for (int64_t base = 0; base + first_slot < n_chunks; base += n_slots * UNR) {   // warp-uniform trip count
         float4 x[UNR][NV];
         int64_t c[UNR];
 #pragma unroll
@@ -237,6 +330,32 @@ qsgd_encode_chunks_kernel(const float *__restrict__ v, int64_t n_chunks, int dim
                 qsgd_store_packed<BITS>(packed, q, pk);
             }
         }
+        if constexpr (DELIVER) {
+            // this iteration's UNR runs of SPB consecutive chunks, read back: norms and packed levels
+            __syncthreads();
+#pragma unroll
+            for (int u = 0; u < UNR; ++u) {
+                const int64_t c0 = base + (int64_t)u * n_slots + (int64_t)blockIdx.x * SPB;
+                if (c0 >= n_chunks) break;
+                const int64_t c1 = min(c0 + SPB, n_chunks);
+                deliver_bytes(R, norm + c0, norm + c1);
+                deliver_bytes(R, static_cast<uint8_t *>(packed) + c0 * dim4 * (BITS / 2),
+                              static_cast<uint8_t *>(packed) + c1 * dim4 * (BITS / 2));
+            }
+        }
+    }
+    if constexpr (DELIVER) {
+        deliver_finish(R, [&] {
+            // the 32-bit words two runs share (4-bit wire, dim / 4 odd: a run boundary falls mid-word),
+            // and a last word that the section ends inside (sent whole: the section is padded to 4 bytes)
+            if (BITS == 4 && (dim4 & 1)) {
+                const int64_t n_runs = (n_chunks + SPB - 1) / SPB;
+                for (int64_t k = 1 + threadIdx.x; k <= n_runs; k += blockDim.x) {
+                    const int64_t b = min(k * SPB, n_chunks) * dim4 * 2;
+                    if (b & 2) deliver_word(R, static_cast<uint8_t *>(packed) + b);
+                }
+            }
+        });
     }
 }
 
@@ -324,12 +443,12 @@ seg_absmax_ranges_kernel(const float *__restrict__ v, int64_t n, const int64_t *
     flush();
 }
 
-template <int BITS, int UN>
+template <int BITS, int UN, bool DELIVER>
 __global__ void __launch_bounds__(256)
 qsgd_quantize_ranges_kernel(const float *__restrict__ v, int64_t n, const int64_t *__restrict__ chunk_start,
                             int n_chunks, float s, int random, const float *__restrict__ uniforms,
                             uint64_t seed, uint64_t offset, const float *__restrict__ norm,
-                            void *__restrict__ packed)
+                            void *__restrict__ packed, const Remote rem)
 {
     pdl_launch_dependents();
     // every CTA owns a contiguous range, its eight warps take the spans of that range in turn (the
@@ -348,6 +467,14 @@ qsgd_quantize_ranges_kernel(const float *__restrict__ v, int64_t n, const int64_
     int cur = -1;
     float nm_cur = 0.0f;
     pdl_wait();
+    if constexpr (DELIVER) {
+        // the per-tensor norms are final once the first pass has completed (atomicMax), and so is the
+        // identity section its rider wrote
+        deliver_ident(rem);
+        if (blockIdx.x == 0)
+            for (int i = threadIdx.x; i < n_chunks; i += 256)
+                remote_st32(rem, const_cast<float *>(norm) + i, __float_as_uint(__ldcg(norm + i)));
+    }
     for (int64_t e0 = e_begin; e0 < e_end; e0 += 8 * span) {
         const int64_t e1 = min(e0 + span, e_end);
         float4 x[UN];
@@ -402,20 +529,63 @@ qsgd_quantize_ranges_kernel(const float *__restrict__ v, int64_t n, const int64_
             qsgd_store_packed<BITS>(packed, i0 >> 2, pk);
         }
     }
+    if constexpr (DELIVER) {
+        // the CTA's packed range (R is a multiple of 4096 elements: interior ends are 16-byte aligned)
+        uint8_t *pb = static_cast<uint8_t *>(packed);
+        const int64_t q_end = (n + 3) >> 2;
+        const int64_t qa = min((int64_t)blockIdx.x * R / 4, q_end), qz = min((int64_t)(blockIdx.x + 1) * R / 4, q_end);
+        __syncthreads();
+        deliver_bytes(rem, pb + qa * (BITS / 2), pb + qz * (BITS / 2));
+        deliver_finish(rem, [&] {
+            if ((q_end * (BITS / 2)) & 3) deliver_word(rem, pb + q_end * (BITS / 2));   // the section ends mid-word
+        });
+    }
 }
 
 int qsgd_wire_bits(int n_bit) { return n_bit <= 2 ? 4 : (n_bit <= 6 ? 8 : 16); }
 
+// The pending remote delivery as the kernels take it.  An identity section to mirror must be the one a
+// rider of the same launch writes (thread i of the grid reads back element i), or one an earlier launch wrote.
+static int device_remote(const Tc2Remote &t, const Rider &rider, Remote *R)
+{
+    GQ_REQUIRE(t.counter != nullptr, "a delivering sign / QSGD encode needs an arrival counter (gq_attach_delivery_counter)");
+    GQ_REQUIRE(rider.n == 0 || t.ident_bytes == 0 || (const void *)rider.out == (const void *)t.ident,
+               "the identity section to deliver is not the one this encode's rider writes");
+    *R = Remote{};
+    R->n = t.n;
+    R->multicast = t.multicast;
+    for (int i = 0; i < 7; ++i) R->delta[i] = i < t.n ? t.delta[i] : 0;
+    R->ident = t.ident;
+    R->ident_bytes = t.ident_bytes;
+    R->done = t.counter;
+    R->n_flag = t.n_flag;
+    for (int i = 0; i < 8; ++i) R->flag[i] = i < t.n_flag ? t.flag[i] : nullptr;
+    R->epoch = t.epoch;
+    return GQ_OK;
+}
+
+// remote: the pending delivery (n == 0: none).  Only the one-launch chunked kernel and the TernGrad range
+// kernels deliver; a call that would take another path returns GQ_ERR_UNSUPPORTED before it launches anything.
 int qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int64_t n_chunks, int dim,
                 int n_bit, int random, const float *uniforms, uint64_t seed, uint64_t offset, float *norm,
-                uint8_t *signs, int32_t *l, void *packed, cudaStream_t st)
+                uint8_t *signs, int32_t *l, void *packed, const Tc2Remote &remote, cudaStream_t st)
 {
-    if (n == 0) return GQ_OK;
+    const bool deliver = remote.n > 0;
     const float s = (float)(1u << n_bit);
     const bool fast_ok = packed && !signs && !l && ((uintptr_t)packed & 15) == 0 && n_chunks < (1ll << 31);
-    if (fast_ok && !chunk_start && dim % 4 == 0 && dim <= 2048) {
+    const bool chunked = fast_ok && !chunk_start && dim % 4 == 0 && dim <= 2048;
+    const bool ranges = fast_ok && chunk_start && ((uintptr_t)grad & 15) == 0;
+    if (deliver && (n == 0 || !(chunked || ranges))) {
+        set_error("a remote delivery is attached, but this QSGD encode takes the generic kernels (packed output only, "
+                  "16-byte aligned, dim %% 4 == 0 and dim <= 2048, or explicit chunk boundaries)");
+        return GQ_ERR_UNSUPPORTED;
+    }
+    if (n == 0) return GQ_OK;
+    if (chunked) {
         // one launch: chunk norms and packed levels from registers
         const Rider rider = take_rider();   // a pending identity copy rides in this launch
+        Remote R = {};
+        if (deliver) GQ_CUDA_INT(device_remote(remote, rider, &R));
         const int b = qsgd_wire_bits(n_bit);
         const int dim4 = dim / 4;
         const int lpc = dim4 <= 8 ? 8 : 32;
@@ -423,8 +593,11 @@ int qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int64_
         const int unr = nv == 1 ? 4 : (nv == 2 ? 2 : 1);
         const int64_t per_block = (int64_t)(256 / lpc) * unr;
         const int grid = grid_for(n_chunks, (int)per_block, 16);
-#define GQ_E(B, NV, LPC, UNR) GQ_CUDA(launch_pdl(qsgd_encode_chunks_kernel<B, NV, LPC, UNR>, dim3(grid), dim3(256), 0, st, \
-                                       grad, n_chunks, dim, s, random, uniforms, seed, offset, norm, packed, rider))
+#define GQ_E(B, NV, LPC, UNR)                                                                                           \
+        GQ_CUDA(deliver ? launch_pdl(qsgd_encode_chunks_kernel<B, NV, LPC, UNR, true>, dim3(grid), dim3(256), 0, st,   \
+                                     grad, n_chunks, dim, s, random, uniforms, seed, offset, norm, packed, rider, R)   \
+                        : launch_pdl(qsgd_encode_chunks_kernel<B, NV, LPC, UNR, false>, dim3(grid), dim3(256), 0, st,  \
+                                     grad, n_chunks, dim, s, random, uniforms, seed, offset, norm, packed, rider, R))
 #define GQ_EB(B)                                                  \
         do {                                                      \
             if (lpc == 8) GQ_E(B, 1, 8, 4);                       \
@@ -443,7 +616,7 @@ int qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int64_
         return GQ_OK;
     }
     GQ_CUDA(cudaMemsetAsync(norm, 0, (size_t)n_chunks * 4, st));
-    if (fast_ok && chunk_start && ((uintptr_t)grad & 15) == 0) {
+    if (ranges) {
         // explicit chunk boundaries (TernGrad): contiguous range per warp, two launches
         // one CTA-contiguous range per CTA and exactly ONE wave: the grid is the number of CTAs that are
         // resident at once (8 per SM asked for 1184 CTAs of which 5 / 4 per SM fit: a second, 60 % full wave)
@@ -457,13 +630,17 @@ int qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int64_
         };
         const int grid_a = one_wave(seg_absmax_ranges_kernel<4>);
         const Rider rider = take_rider();   // a pending identity copy rides in the first pass
+        Remote R = {};   // the second pass delivers (the norms are final only after the first)
+        if (deliver) GQ_CUDA_INT(device_remote(remote, rider, &R));
         GQ_CUDA(launch_pdl(seg_absmax_ranges_kernel<4>, dim3(grid_a), dim3(256), 0, st, grad, n, chunk_start, (int)n_chunks,
                            reinterpret_cast<uint32_t *>(norm), rider));
-#define GQ_R(B) GQ_CUDA(launch_pdl(qsgd_quantize_ranges_kernel<B, 4>, dim3(one_wave(qsgd_quantize_ranges_kernel<B, 4>)), dim3(256), 0, st, grad, n, chunk_start, \
-                                   (int)n_chunks, s, random, uniforms, seed, offset, (const float *)norm, packed))
-        if (b == 4) GQ_R(4);
-        else if (b == 8) GQ_R(8);
-        else GQ_R(16);
+#define GQ_R(B, D) GQ_CUDA(launch_pdl(qsgd_quantize_ranges_kernel<B, 4, D>, dim3(one_wave(qsgd_quantize_ranges_kernel<B, 4, D>)), dim3(256), 0, st, \
+                                      grad, n, chunk_start, (int)n_chunks, s, random, uniforms, seed, offset, (const float *)norm, packed, R))
+#define GQ_RB(B) do { if (deliver) GQ_R(B, true); else GQ_R(B, false); } while (0)
+        if (b == 4) GQ_RB(4);
+        else if (b == 8) GQ_RB(8);
+        else GQ_RB(16);
+#undef GQ_RB
 #undef GQ_R
         GQ_LAUNCH_CHECK("qsgd_quantize_ranges");
         return GQ_OK;
@@ -541,18 +718,19 @@ qsgd_decode_reduce_kernel(const float *__restrict__ norm, const void *__restrict
 // Fast decode-and-reduce: 8 consecutive elements per thread (one 32 / 64 / 128-bit word of packed
 // levels per user, two float4 stores), the chunk index from one 32-bit division per thread (or the
 // thread's cached segment), "/ s" and a power-of-two "/ U" as exact multiplications by 2^-k.
-template <int BITS, int U_>   // U_ > 0: number of users at compile time
+template <int BITS, int U_, bool WAIT>   // U_ > 0: number of users at compile time
 __global__ void __launch_bounds__(256)
 qsgd_decode_reduce8_kernel(const float *__restrict__ norm, const void *__restrict__ packed, int64_t user_stride,
                            int n_users_rt, int64_t n, const int64_t *__restrict__ chunk_start, int n_chunks,
                            uint32_t dim, float inv_s, float inv_u, float div_u, int accumulate,
-                           float *__restrict__ out, const Rider rider)
+                           float *__restrict__ out, const Rider rider, const PeerWait wait)
 {
     pdl_launch_dependents();
     const int n_users = U_ > 0 ? U_ : n_users_rt;
     const int64_t n8 = n >> 3;
     SegCache sc;
     pdl_wait();
+    wait_prologue<WAIT>(wait);   // the peers' delivery flags, before any record byte is read
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
     if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) {
         // the last n % 8 elements, one by one
@@ -604,22 +782,22 @@ qsgd_decode_reduce8_kernel(const float *__restrict__ norm, const void *__restric
             const float *nu = reinterpret_cast<const float *>(reinterpret_cast<const char *>(norm) + u * user_stride);
             uint32_t pk[8];
             if (BITS == 4) {
-                const uint32_t w = __ldg(reinterpret_cast<const uint32_t *>(pu) + q);
+                const uint32_t w = ld_rec<WAIT>(reinterpret_cast<const uint32_t *>(pu) + q);
 #pragma unroll
                 for (int t = 0; t < 8; ++t) pk[t] = (w >> (4 * t)) & 15u;
             } else if (BITS == 8) {
-                const uint2 w = __ldg(reinterpret_cast<const uint2 *>(pu) + q);
+                const uint2 w = ld_rec<WAIT>(reinterpret_cast<const uint2 *>(pu) + q);
 #pragma unroll
                 for (int t = 0; t < 4; ++t) { pk[t] = (w.x >> (8 * t)) & 255u; pk[4 + t] = (w.y >> (8 * t)) & 255u; }
             } else {
-                const uint4 w = __ldg(reinterpret_cast<const uint4 *>(pu) + q);
+                const uint4 w = ld_rec<WAIT>(reinterpret_cast<const uint4 *>(pu) + q);
                 pk[0] = w.x & 0xffffu; pk[1] = w.x >> 16; pk[2] = w.y & 0xffffu; pk[3] = w.y >> 16;
                 pk[4] = w.z & 0xffffu; pk[5] = w.z >> 16; pk[6] = w.w & 0xffffu; pk[7] = w.w >> 16;
             }
-            const float nm0 = __ldg(nu + m[0]);
+            const float nm0 = ld_rec<WAIT>(nu + m[0]);
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
-                const float nm = uni ? nm0 : __ldg(nu + m[t]);
+                const float nm = uni ? nm0 : ld_rec<WAIT>(nu + m[t]);
                 const uint32_t sg = pk[t] >> (BITS - 1);
                 const float lf = (float)(int)(pk[t] & ((1u << (BITS - 1)) - 1u));
                 // (float(l) * (2 * sign - 1)) * norm / s, qsgd_compressor.py:69-70
@@ -656,11 +834,16 @@ static void mean_factors(int mean, int n_users, float *inv_u, float *div_u)
     else *div_u = (float)n_users;
 }
 
+// wait: the peers' delivery flags to poll first (n == 0: none); in the fast kernel's prologue, else in a
+// one-warp kernel of its own
 int qsgd_decode_reduce(const float *norm, const void *packed, int64_t user_stride, int n_users,
                        int64_t n, const int64_t *chunk_start, int64_t n_chunks, int dim, int n_bit,
-                       int mean, int accumulate, float *out, cudaStream_t st)
+                       int mean, int accumulate, float *out, const PeerWait &wait, cudaStream_t st)
 {
-    if (n == 0) return GQ_OK;
+    if (n == 0) {
+        set_wait(wait);
+        return flush_wait(st);
+    }
     const float s = (float)(1u << n_bit);
     const int bits = qsgd_wire_bits(n_bit);
     const int64_t n8 = n / 8;
@@ -670,8 +853,9 @@ int qsgd_decode_reduce(const float *norm, const void *packed, int64_t user_strid
         mean_factors(mean, n_users, &inv_u, &div_u);
         const int grid8 = grid_for(n8 + 1, 256, 16);
         const Rider rider = take_rider();   // a pending identity reduction rides in this launch
-#define GQ_D8(B, UU) GQ_CUDA(launch_pdl(qsgd_decode_reduce8_kernel<B, UU>, dim3(grid8), dim3(256), 0, st, norm, packed, user_stride, \
-                                        n_users, n, chunk_start, (int)n_chunks, (uint32_t)(dim > 0 ? dim : 1), 1.0f / s, inv_u, div_u, accumulate, out, rider))
+#define GQ_D8W(B, UU, W) GQ_CUDA(launch_pdl(qsgd_decode_reduce8_kernel<B, UU, W>, dim3(grid8), dim3(256), 0, st, norm, packed, user_stride, \
+                                            n_users, n, chunk_start, (int)n_chunks, (uint32_t)(dim > 0 ? dim : 1), 1.0f / s, inv_u, div_u, accumulate, out, rider, wait))
+#define GQ_D8(B, UU) do { if (wait.n > 0) GQ_D8W(B, UU, true); else GQ_D8W(B, UU, false); } while (0)
 #define GQ_D8B(B) do { if (n_users == 1) GQ_D8(B, 1); else if (n_users == 2) GQ_D8(B, 2); else if (n_users == 4) GQ_D8(B, 4); \
                        else if (n_users == 8) GQ_D8(B, 8); else GQ_D8(B, 0); } while (0)
         if (bits == 4) GQ_D8B(4);
@@ -679,9 +863,12 @@ int qsgd_decode_reduce(const float *norm, const void *packed, int64_t user_strid
         else GQ_D8B(16);
 #undef GQ_D8B
 #undef GQ_D8
+#undef GQ_D8W
         GQ_LAUNCH_CHECK("qsgd_decode_reduce8");
         return GQ_OK;
     }
+    set_wait(wait);
+    GQ_CUDA_INT(flush_wait(st));
     const int grid = grid_for((n + 3) / 4, 256);
 #define GQ_D(B) qsgd_decode_reduce_kernel<B><<<grid, 256, 0, st>>>(norm, packed, user_stride, n_users, n, chunk_start, n_chunks, dim, s, mean, accumulate, out)
     if (bits == 4) GQ_D(4);
@@ -756,10 +943,11 @@ sign_encode_kernel(const float *__restrict__ v, int64_t n, float *__restrict__ o
 // user (one coalesced 128-byte request per user), the words are redistributed by shuffles so that lane
 // L produces the float4 groups L, 32 + L, 64 + L, 96 + L of the tile: four fully coalesced 512-byte
 // stores (a thread writing its own 16 consecutive elements would put half-sector writes on L2).
-template <int U_>
+template <int U_, bool WAIT>
 __global__ void __launch_bounds__(256)
 sign_decode_reduce_kernel(const uint8_t *__restrict__ packed, int64_t user_stride, int n_users_rt,
-                          int64_t n, float inv_u, float div_u, int accumulate, float *__restrict__ out, const Rider rider)
+                          int64_t n, float inv_u, float div_u, int accumulate, float *__restrict__ out, const Rider rider,
+                          const PeerWait wait)
 {
     pdl_launch_dependents();
     const int n_users = U_ > 0 ? U_ : n_users_rt;
@@ -768,6 +956,7 @@ sign_decode_reduce_kernel(const uint8_t *__restrict__ packed, int64_t user_strid
     const bool aligned = ((reinterpret_cast<uintptr_t>(out) & 15) == 0) && ((user_stride & 3) == 0) &&
                          ((reinterpret_cast<uintptr_t>(packed) & 3) == 0);
     pdl_wait();
+    wait_prologue<WAIT>(wait);   // the peers' delivery flags, before any record byte is read
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
     for (int64_t tile = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5); tile < n_tiles; tile += (int64_t)gridDim.x * 8) {
         const int64_t e0 = tile * 512;
@@ -777,7 +966,7 @@ sign_decode_reduce_kernel(const uint8_t *__restrict__ packed, int64_t user_strid
             const uint8_t *pu = packed + u * user_stride + (e0 >> 2);
             uint32_t w = 0u;
             if (full) {
-                w = __ldg(reinterpret_cast<const uint32_t *>(pu) + lane);
+                w = ld_rec<WAIT>(reinterpret_cast<const uint32_t *>(pu) + lane);
             } else {
                 for (int k = 0; k < 4; ++k)
                     if (e0 + 16 * lane + 4 * k < n) w |= (uint32_t)pu[4 * lane + k] << (8 * k);
@@ -832,13 +1021,15 @@ sign_decode_reduce_kernel(const uint8_t *__restrict__ packed, int64_t user_strid
 // same digit code as the 2-bit form (0 -> 0, 1 -> +1, 2 -> -1): 1.6 bits per element instead of 2.
 // A thread owns 20 consecutive elements = one 32-bit word of the wire (little-endian bytes); the
 // section holds ceil(n / 20) words, elements past n encode as 0.
+template <bool DELIVER>
 __global__ void __launch_bounds__(256)
-sign_encode_t5_kernel(const float *__restrict__ v, int64_t n, uint32_t *__restrict__ packed, const Rider rider)
+sign_encode_t5_kernel(const float *__restrict__ v, int64_t n, uint32_t *__restrict__ packed, const Rider rider, const Remote R)
 {
     pdl_launch_dependents();
     const int64_t n_words = (n + 19) / 20;
     pdl_wait();
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
+    if constexpr (DELIVER) deliver_ident(R);
     for (int64_t w = (int64_t)blockIdx.x * 256 + threadIdx.x; w < n_words; w += (int64_t)gridDim.x * 256) {
         const int64_t i0 = w * 20;
         float x[20];
@@ -864,16 +1055,19 @@ sign_encode_t5_kernel(const float *__restrict__ v, int64_t n, uint32_t *__restri
             word = (word << 8) | byte;
         }
         packed[w] = word;
+        if constexpr (DELIVER) remote_st32(R, packed + w, word);
     }
+    if constexpr (DELIVER) deliver_finish(R, [] {});
 }
 
 // A warp decodes 640 elements at a time: lane L takes word L of every user (one coalesced 128-byte
 // request per user), sums its 20 values in user order, and the warp transposes the 640 results through
 // shared memory so that the stores are five fully coalesced 512-byte rows (see sign_decode_reduce_kernel).
-template <int U_>
+template <int U_, bool WAIT>
 __global__ void __launch_bounds__(256)
 sign_decode_reduce_t5_kernel(const uint32_t *__restrict__ packed, int64_t user_stride_words, int n_users_rt,
-                             int64_t n, float inv_u, float div_u, int accumulate, float *__restrict__ out, const Rider rider)
+                             int64_t n, float inv_u, float div_u, int accumulate, float *__restrict__ out, const Rider rider,
+                             const PeerWait wait)
 {
     __shared__ float4 s_t[8][160];   // per warp: 640 floats
     pdl_launch_dependents();
@@ -883,13 +1077,14 @@ sign_decode_reduce_t5_kernel(const uint32_t *__restrict__ packed, int64_t user_s
     const int64_t n_words = (n + 19) / 20;
     const bool aligned = (reinterpret_cast<uintptr_t>(out) & 15) == 0;
     pdl_wait();
+    wait_prologue<WAIT>(wait);   // the peers' delivery flags, before any record byte is read
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
     for (int64_t tile = (int64_t)blockIdx.x * 8 + warp; tile < n_tiles; tile += (int64_t)gridDim.x * 8) {
         const int64_t e0 = tile * 640;
         const int64_t w = tile * 32 + lane;
         float acc[20];
         for (int u = 0; u < n_users; ++u) {
-            uint32_t word = (w < n_words) ? __ldg(packed + u * user_stride_words + w) : 0u;
+            uint32_t word = (w < n_words) ? ld_rec<WAIT>(packed + u * user_stride_words + w) : 0u;
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
                 uint32_t by = word & 0xffu;
@@ -942,31 +1137,40 @@ sign_decode_reduce_t5_kernel(const uint32_t *__restrict__ packed, int64_t user_s
     }
 }
 
-int sign_encode_t5(const float *grad, int64_t n, uint32_t *packed, cudaStream_t st)
+int sign_encode_t5(const float *grad, int64_t n, uint32_t *packed, const Tc2Remote &remote, cudaStream_t st)
 {
     if (n == 0) return GQ_OK;
     const Rider rider = take_rider();   // a pending identity copy rides in this launch
-    GQ_CUDA(launch_pdl(sign_encode_t5_kernel, dim3(grid_for((n + 19) / 20, 256, 16)), dim3(256), 0, st, grad, n, packed, rider));
+    Remote R = {};
+    if (remote.n > 0) GQ_CUDA_INT(device_remote(remote, rider, &R));
+    const dim3 grid(grid_for((n + 19) / 20, 256, 16));
+    GQ_CUDA(remote.n > 0 ? launch_pdl(sign_encode_t5_kernel<true>, grid, dim3(256), 0, st, grad, n, packed, rider, R)
+                         : launch_pdl(sign_encode_t5_kernel<false>, grid, dim3(256), 0, st, grad, n, packed, rider, R));
     GQ_LAUNCH_CHECK("sign_encode_t5");
     return GQ_OK;
 }
 
 int sign_decode_reduce_t5(const uint32_t *packed, int64_t user_stride_words, int n_users, int64_t n, int mean,
-                          int accumulate, float *out, cudaStream_t st)
+                          int accumulate, float *out, const PeerWait &wait, cudaStream_t st)
 {
-    if (n == 0) return GQ_OK;
+    if (n == 0) {
+        set_wait(wait);
+        return flush_wait(st);
+    }
     float inv_u, div_u;
     mean_factors(mean, n_users, &inv_u, &div_u);
     const int grid = grid_for((n + 639) / 640, 8, 8);
     const Rider rider = take_rider();   // a pending identity reduction rides in this launch
-#define GQ_S(UU) GQ_CUDA(launch_pdl(sign_decode_reduce_t5_kernel<UU>, dim3(grid), dim3(256), 0, st, packed, user_stride_words, \
-                                    n_users, n, inv_u, div_u, accumulate, out, rider))
+#define GQ_SW(UU, W) GQ_CUDA(launch_pdl(sign_decode_reduce_t5_kernel<UU, W>, dim3(grid), dim3(256), 0, st, packed, user_stride_words, \
+                                        n_users, n, inv_u, div_u, accumulate, out, rider, wait))
+#define GQ_S(UU) do { if (wait.n > 0) GQ_SW(UU, true); else GQ_SW(UU, false); } while (0)
     if (n_users == 1) GQ_S(1);
     else if (n_users == 2) GQ_S(2);
     else if (n_users == 4) GQ_S(4);
     else if (n_users == 8) GQ_S(8);
     else GQ_S(0);
 #undef GQ_S
+#undef GQ_SW
     GQ_LAUNCH_CHECK("sign_decode_reduce_t5");
     return GQ_OK;
 }
@@ -974,13 +1178,15 @@ int sign_decode_reduce_t5(const uint32_t *packed, int64_t user_stride_words, int
 // packed output only (the fused plan): a thread owns 16 consecutive elements = one 32-bit word of the
 // wire -- four 16-byte loads in flight per thread and a coalesced 128-byte store per warp instead of 32
 // single bytes (21.0 -> see DESIGN.md section 8)
+template <bool DELIVER>
 __global__ void __launch_bounds__(256)
-sign_encode_words_kernel(const float *__restrict__ v, int64_t n, uint32_t *__restrict__ packed, const Rider rider)
+sign_encode_words_kernel(const float *__restrict__ v, int64_t n, uint32_t *__restrict__ packed, const Rider rider, const Remote R)
 {
     pdl_launch_dependents();
     const int64_t n_words = n / 16;   // whole words; the ragged tail goes through sign_encode_kernel
     pdl_wait();
     rider_run(rider, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);   // identity tensors ride along
+    if constexpr (DELIVER) deliver_ident(R);
     for (int64_t w = (int64_t)blockIdx.x * 256 + threadIdx.x; w < n_words; w += (int64_t)gridDim.x * 256) {
         float4 t[4];
 #pragma unroll
@@ -994,17 +1200,53 @@ sign_encode_words_kernel(const float *__restrict__ v, int64_t n, uint32_t *__res
                 word |= ((x[k] > 0.0f ? 1u : 0u) | (x[k] < 0.0f ? 2u : 0u)) << (8 * q + 2 * k);
         }
         packed[w] = word;
+        if constexpr (DELIVER) remote_st32(R, packed + w, word);
+    }
+    if constexpr (DELIVER) {
+        // a delivering launch encodes the ragged tail itself (at most 15 elements: the bytes that
+        // sign_encode_kernel would write), then sends that word whole -- the section is padded to 4 bytes
+        const int64_t done = n_words * 16;
+        if (done < n && blockIdx.x == gridDim.x - 1 && threadIdx.x == 0) {
+            uint8_t *pb = reinterpret_cast<uint8_t *>(packed + n_words);
+            for (int b = 0; 4 * b < n - done; ++b) {
+                uint32_t byte = 0u;
+                for (int k = 0; k < 4; ++k) {
+                    const float x = (done + 4 * b + k < n) ? v[done + 4 * b + k] : 0.0f;
+                    byte |= ((x > 0.0f ? 1u : 0u) | (x < 0.0f ? 2u : 0u)) << (2 * k);
+                }
+                pb[b] = (uint8_t)byte;
+            }
+            deliver_word(R, pb);
+        }
+        deliver_finish(R, [] {});
     }
 }
 
-int sign_encode(const float *grad, int64_t n, float *out_f32, uint8_t *packed, cudaStream_t st)
+// remote: the pending delivery (n == 0: none), which only the packed-words kernel makes; a call that would
+// take the other kernel returns GQ_ERR_UNSUPPORTED before it launches anything
+int sign_encode(const float *grad, int64_t n, float *out_f32, uint8_t *packed, const Tc2Remote &remote, cudaStream_t st)
 {
+    const bool words = !out_f32 && packed && ((uintptr_t)packed & 3) == 0;
+    if (remote.n > 0) {
+        if (!words || n == 0) {
+            set_error("a remote delivery is attached, but this sign encode is not the packed-words kernel "
+                      "(packed output only, 4-byte aligned, n > 0)");
+            return GQ_ERR_UNSUPPORTED;
+        }
+        const Rider rider = take_rider();   // a pending identity copy rides in this launch
+        Remote R = {};
+        GQ_CUDA_INT(device_remote(remote, rider, &R));
+        GQ_CUDA(launch_pdl(sign_encode_words_kernel<true>, dim3(grid_for(n / 16 + 1, 256, 16)), dim3(256), 0, st, grad, n,
+                           reinterpret_cast<uint32_t *>(packed), rider, R));
+        GQ_LAUNCH_CHECK("sign_encode");
+        return GQ_OK;
+    }
     if (n == 0) return GQ_OK;
-    if (!out_f32 && packed && ((uintptr_t)packed & 3) == 0 && n >= 16) {
+    if (words && n >= 16) {
         const int64_t n_words = n / 16;
         const Rider rider = take_rider();   // a pending identity copy rides in this launch
-        GQ_CUDA(launch_pdl(sign_encode_words_kernel, dim3(grid_for(n_words, 256, 16)), dim3(256), 0, st, grad, n,
-                           reinterpret_cast<uint32_t *>(packed), rider));
+        GQ_CUDA(launch_pdl(sign_encode_words_kernel<false>, dim3(grid_for(n_words, 256, 16)), dim3(256), 0, st, grad, n,
+                           reinterpret_cast<uint32_t *>(packed), rider, Remote{}));
         const int64_t done = n_words * 16;
         if (done < n)   // at most 15 elements
             sign_encode_kernel<<<1, 32, 0, st>>>(grad + done, n - done, nullptr, packed + done / 4);
@@ -1017,21 +1259,26 @@ int sign_encode(const float *grad, int64_t n, float *out_f32, uint8_t *packed, c
 }
 
 int sign_decode_reduce(const uint8_t *packed, int64_t user_stride, int n_users, int64_t n, int mean,
-                       int accumulate, float *out, cudaStream_t st)
+                       int accumulate, float *out, const PeerWait &wait, cudaStream_t st)
 {
-    if (n == 0) return GQ_OK;
+    if (n == 0) {
+        set_wait(wait);
+        return flush_wait(st);
+    }
     float inv_u, div_u;
     mean_factors(mean, n_users, &inv_u, &div_u);
     const int grid = grid_for((n + 511) / 512, 8, 16);
     const Rider rider = take_rider();   // a pending identity reduction rides in this launch
-#define GQ_S(UU) GQ_CUDA(launch_pdl(sign_decode_reduce_kernel<UU>, dim3(grid), dim3(256), 0, st, packed, user_stride, n_users, n, \
-                                    inv_u, div_u, accumulate, out, rider))
+#define GQ_SW(UU, W) GQ_CUDA(launch_pdl(sign_decode_reduce_kernel<UU, W>, dim3(grid), dim3(256), 0, st, packed, user_stride, n_users, n, \
+                                        inv_u, div_u, accumulate, out, rider, wait))
+#define GQ_S(UU) do { if (wait.n > 0) GQ_SW(UU, true); else GQ_SW(UU, false); } while (0)
     if (n_users == 1) GQ_S(1);
     else if (n_users == 2) GQ_S(2);
     else if (n_users == 4) GQ_S(4);
     else if (n_users == 8) GQ_S(8);
     else GQ_S(0);
 #undef GQ_S
+#undef GQ_SW
     GQ_LAUNCH_CHECK("sign_decode_reduce");
     return GQ_OK;
 }
@@ -1050,6 +1297,7 @@ int gq_qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int
                    gq_stream_t stream)
 {
     const Rider pending = take_rider();   // consumed first: an early error return must not leave it armed
+    const Tc2Remote remote = take_remote();   // likewise the pending delivery to the peers
     GQ_REQUIRE(n >= 0 && n_chunks >= 0, "negative size");
     GQ_REQUIRE(n_bit >= 1 && n_bit <= 14, "n_bit %d out of range 1..14", n_bit);
     GQ_REQUIRE(chunk_start || (dim >= 1 && n_chunks * (int64_t)dim == n),
@@ -1059,7 +1307,7 @@ int gq_qsgd_encode(const float *grad, int64_t n, const int64_t *chunk_start, int
     GQ_REQUIRE(((uintptr_t)grad & 15) == 0, "gradient must be 16-byte aligned");
     set_rider(pending);
     const int e = qsgd_encode(grad, n, chunk_start, n_chunks, dim, n_bit, random, uniforms, philox_seed,
-                              philox_offset, norm, signs, l, packed, as_stream(stream));
+                              philox_offset, norm, signs, l, packed, remote, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));   // no-op when the encode kernel carried it
@@ -1070,13 +1318,14 @@ int gq_qsgd_decode_reduce(const float *norm, const void *packed, int64_t user_st
                           int mean, int accumulate, float *out, gq_stream_t stream)
 {
     const Rider pending = take_rider();
+    const PeerWait wait = take_wait();
     GQ_REQUIRE(n >= 0 && n_users >= 1, "bad sizes");
     GQ_REQUIRE(n_bit >= 1 && n_bit <= 14, "n_bit %d out of range 1..14", n_bit);
     GQ_REQUIRE(chunk_start || (dim >= 1 && n_chunks * (int64_t)dim == n), "n != n_chunks * dim");
     GQ_REQUIRE(n == 0 || (norm && packed && out), "null pointer");
     set_rider(pending);
     const int e = qsgd_decode_reduce(norm, packed, user_stride_bytes, n_users, n, chunk_start, n_chunks, dim,
-                                     n_bit, mean, accumulate, out, as_stream(stream));
+                                     n_bit, mean, accumulate, out, wait, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));
@@ -1096,11 +1345,12 @@ int gq_qsgd_decode_unpacked(const float *norm, const uint8_t *signs, const int32
 int gq_sign_encode(const float *grad, int64_t n, float *out_f32, uint8_t *packed, gq_stream_t stream)
 {
     const Rider pending = take_rider();
+    const Tc2Remote remote = take_remote();
     GQ_REQUIRE(n >= 0 && (n == 0 || grad), "bad arguments");
     GQ_REQUIRE(out_f32 || packed, "need at least one output");
     GQ_REQUIRE(((uintptr_t)grad & 15) == 0, "gradient must be 16-byte aligned");
     set_rider(pending);
-    const int e = sign_encode(grad, n, out_f32, packed, as_stream(stream));
+    const int e = sign_encode(grad, n, out_f32, packed, remote, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));
@@ -1110,9 +1360,10 @@ int gq_sign_decode_reduce(const uint8_t *packed, int64_t user_stride_bytes, int 
                           int mean, int accumulate, float *out, gq_stream_t stream)
 {
     const Rider pending = take_rider();
+    const PeerWait wait = take_wait();
     GQ_REQUIRE(n >= 0 && n_users >= 1 && (n == 0 || (packed && out)), "bad arguments");
     set_rider(pending);
-    const int e = sign_decode_reduce(packed, user_stride_bytes, n_users, n, mean, accumulate, out, as_stream(stream));
+    const int e = sign_decode_reduce(packed, user_stride_bytes, n_users, n, mean, accumulate, out, wait, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));
@@ -1123,10 +1374,15 @@ int64_t gq_sign_t5_bytes(int64_t n) { return n <= 0 ? 0 : (n + 19) / 20 * 4; }
 int gq_sign_encode_t5(const float *grad, int64_t n, void *packed, gq_stream_t stream)
 {
     const Rider pending = take_rider();
+    const Tc2Remote remote = take_remote();
     GQ_REQUIRE(n >= 0 && (n == 0 || (grad && packed)), "bad arguments");
     GQ_REQUIRE(((uintptr_t)grad & 15) == 0 && ((uintptr_t)packed & 3) == 0, "gradient 16-byte, wire 4-byte aligned");
+    if (remote.n > 0 && n == 0) {
+        set_error("a remote delivery is attached to an empty sign encode");
+        return GQ_ERR_UNSUPPORTED;
+    }
     set_rider(pending);
-    const int e = sign_encode_t5(grad, n, reinterpret_cast<uint32_t *>(packed), as_stream(stream));
+    const int e = sign_encode_t5(grad, n, reinterpret_cast<uint32_t *>(packed), remote, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));
@@ -1136,11 +1392,12 @@ int gq_sign_decode_reduce_t5(const void *packed, int64_t user_stride_bytes, int 
                              int accumulate, float *out, gq_stream_t stream)
 {
     const Rider pending = take_rider();
+    const PeerWait wait = take_wait();
     GQ_REQUIRE(n >= 0 && n_users >= 1 && (n == 0 || (packed && out)), "bad arguments");
     GQ_REQUIRE(((uintptr_t)packed & 3) == 0 && (user_stride_bytes & 3) == 0, "wire sections are 4-byte aligned");
     set_rider(pending);
     const int e = sign_decode_reduce_t5(reinterpret_cast<const uint32_t *>(packed), user_stride_bytes / 4, n_users, n, mean,
-                                        accumulate, out, as_stream(stream));
+                                        accumulate, out, wait, as_stream(stream));
     const Rider left = take_rider();
     if (e) return e;
     return launch_rider(left, as_stream(stream));

@@ -591,6 +591,10 @@ int gq_topk_select(const float *grad, int64_t n, const int64_t *seg_start, const
                    void *workspace, size_t workspace_bytes, gq_stream_t stream)
 {
     const Rider pending = take_rider();   // consumed first: an early error return must not leave it armed
+    if (take_remote().n > 0) {            // the record is written by the last of ten launches: no delivery
+        set_error("a remote delivery is attached, but top-k has no delivering encode");
+        return GQ_ERR_UNSUPPORTED;
+    }
     GQ_REQUIRE(n >= 0 && n_seg >= 1, "bad sizes");
     GQ_REQUIRE(n < ((int64_t)1 << 31), "top-k group larger than 2^31 elements");
     GQ_REQUIRE(grad && seg_start && k, "null pointer");

@@ -384,7 +384,8 @@ class FusedPlan:
         return out, pos
 
     # --------------------------------------------------------------- encode ---
-    def encode(self, user, src=None, uniforms=None, rng_user=None, shared_rng=False, part=None, defer_levels=False):
+    def encode(self, user, src=None, uniforms=None, rng_user=None, shared_rng=False, part=None, defer_levels=False,
+               delivery=None):
         """Compress the arena (or `src`, laid out like it) into records[user].
         rng_user: logical user whose Philox stream the stochastic rounding draws from (default: the
         record row); shared_rng: the rank-independent stream instead (second phase of --two-phase).
@@ -395,7 +396,13 @@ class FusedPlan:
         row -- completes it first with the stand-alone quantizer.  The bytes are the same either way.
         Launches: HSQ 2 per group on the tcgen05 path (search, quantize; 3 with the separate init
         kernel of the exact path), QSGD 1 (chunked) or 3, sign 1, top-k 10; the copy of the identity tensors rides
-        in the first HSQ group's first kernel (1 launch of its own when there is no HSQ group)."""
+        in the first HSQ group's first kernel (1 launch of its own when there is no HSQ group).
+        delivery: PeerRecords.attach_delivery's re-attaching function, for an encode of several launches (one
+        per group): every launch delivers its own sections, the carrier's the identity section too, and only
+        the last one announces the step's epoch.  Its kernels run in stream order with programmatic
+        dependent launch: a launch's CTAs pass griddepcontrol.wait, i.e. the previous launch has completed
+        and its remote stores are performed, before they arrive on the counter, so the last launch's
+        system-scope release of the flag comes after every earlier launch's remote stores."""
         src = self.arena if src is None else src
         src_ptr = src if isinstance(src, int) else src.data_ptr()   # tensor or raw device address
         rng_user = user if rng_user is None else rng_user
@@ -411,9 +418,12 @@ class FusedPlan:
         ident, carrier = self._rider_pair()
         if part is not None and not hasattr(self, "n_parts"):
             raise _lib.GQError("encode(part=...) needs make_parts() first")
+        last = ([g for g in self.groups if self._launches_in(g, part)] or [None])[-1]
         for g in self.groups:
             gp = src_ptr + g.arena_off * 4
             r = None if uniforms is None else uniforms.get(id(g))
+            if delivery is not None and self._launches_in(g, part):
+                delivery(announce=g is last, ident=g is carrier)
             if part is not None:
                 if g.kind == "hsq" and getattr(g, "part_cuts", None) is not None:
                     pr = self._part_range(g, part)
@@ -477,6 +487,16 @@ class FusedPlan:
                 if g.n and carrier is None:   # a plain copy of the raw fp32 tensors into the record
                     _lib.call("gq_f32_reduce_users", gp, 0, 1, g.n, 0, 0, base + g.raw_off, st)
 
+    def _launches_in(self, g, part):
+        """Does group g launch a codec kernel in encode(part=part) / decode(part=part)?"""
+        if g.kind == "identity":
+            return False
+        if part is None:
+            return True
+        if g.kind == "hsq" and getattr(g, "part_cuts", None) is not None:
+            return self._part_range(g, part) is not None
+        return part == 0
+
     def _rider_pair(self, n_users=1):
         """(identity group, group whose first kernel carries the identity tensors' copy / reduction) or
         (None, None).  Carriers: HSQ, the one-launch sign / QSGD kernels, top-k's setup / fill kernels (their C entry points consume
@@ -506,10 +526,26 @@ class FusedPlan:
                 return False
         return True
 
+    def supports_p2p(self):
+        """The peer-to-peer exchange (PSQuantizer push and gather, RingQuantizer) handles this plan: every
+        plan supports_scattered() accepts, and plans whose compressed groups are all sign groups or all
+        QSGD / TernGrad groups.  Top-k keeps the NCCL exchange."""
+        if self.supports_scattered():
+            return True
+        kinds = {g.kind for g in self.groups if g.kind != "identity"}
+        return kinds == {"sign"} or kinds == {"qsgd"}
+
     def supports_fused_delivery(self):
-        """The one-launch tcgen05 encode can deliver the record to the peers itself when the plan is a
-        single HSQ group with d = 8, 16 or 32, K = 256 and uint8 codes and levels, plus identity."""
+        """The encode kernels can deliver the record to the peers themselves: a single HSQ group on the
+        one-launch tcgen05 encode (d = 8, 16 or 32, K = 256, uint8 codes and levels), or sign groups, or
+        QSGD / TernGrad groups that all take the one-launch chunked kernel (dim % 4 == 0, dim <= 2048) or
+        the TernGrad range kernels -- plus identity."""
         import os
+        comp = [g for g in self.groups if g.kind != "identity"]
+        if comp and all(g.kind == "sign" for g in comp):
+            return True
+        if comp and all(g.kind == "qsgd" for g in comp):
+            return all(g.dim == 0 or (g.dim % 4 == 0 and g.dim <= 2048) for g in comp)
         if os.environ.get("GQ_TC_V", "2") == "1" or self.algo == _lib.ALGO_EXACT:
             return False
         hsq = [g for g in self.groups if g.kind != "identity"]
@@ -553,10 +589,12 @@ class FusedPlan:
         return all(g.kind != "topk" for g in self.groups)
 
     def decode(self, first_user=0, n_users=None, mean=True, accumulate=False, out=None,
-               base_ptr=None, user_offsets=None, part=None):
+               base_ptr=None, user_offsets=None, part=None, wait=None):
         """out (arena layout) = [out +] reduce over records[first_user : first_user+n_users].
         base_ptr / user_offsets (ctypes int64 array): user 0's record address and every user's byte
-        offset from it, for records that live in different buffers (peer-to-peer exchange)."""
+        offset from it, for records that live in different buffers (peer-to-peer exchange).
+        wait: PeerRecords.attach_wait's re-attaching function: every decode launch waits for the peers'
+        delivery flags itself before it reads a record byte."""
         out = self.arena if out is None else out
         n_users = self.n_users if n_users is None else n_users
         st = _lib.stream()
@@ -587,6 +625,8 @@ class FusedPlan:
         stride = self.record_bytes
         for g in self.groups:
             op = out.data_ptr() + g.arena_off * 4
+            if wait is not None and self._launches_in(g, part):
+                wait()
             if part is not None:
                 if g.kind == "hsq" and getattr(g, "part_cuts", None) is not None:
                     pr = self._part_range(g, part)

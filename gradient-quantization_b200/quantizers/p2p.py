@@ -29,6 +29,7 @@ class _CudaBuffer:
 
 class PeerRecords:
     FLAG_BYTES = 256
+    COUNTER_OFFSET = 64   # in the local flag area: the arrival counter of the delivering sign / QSGD encodes
 
     def __init__(self, record_bytes, rank, world, device):
         assert world <= 8
@@ -112,10 +113,31 @@ class PeerRecords:
     def parity(self):
         return self.step & 1
 
+    def _delivery(self, plan, deltas, mc, flag_ranks, epoch, with_ident):
+        """Attach a delivery now and return a function that attaches it again: deliver(announce, ident)
+        before every launch of an encode made of several calls (FusedPlan.encode), so that each launch
+        delivers its own sections and only the last one announces `epoch`."""
+        local = self._addr(self.rank, self.rank)
+        g_id = next((g for g in plan.groups if g.kind == "identity" and g.n), None) if with_ident else None
+        delta_arr = (ctypes.c_int64 * len(deltas))(*deltas)
+        flags = (ctypes.c_void_p * len(flag_ranks))(*[int(self._flag_ptrs[r]) + 4 * self.rank for r in flag_ranks])
+        counter = int(self._flag_ptrs[self.rank]) + self.COUNTER_OFFSET
+
+        def deliver(announce=True, ident=True):
+            g = g_id if ident else None
+            _lib.call("gq_attach_remote_record", len(deltas), mc, delta_arr, local + g.raw_off if g is not None else None,
+                      (g.n * 4 + 15) // 16 * 16 if g is not None else 0, ctypes.cast(flags, ctypes.c_void_p),
+                      len(flag_ranks) if announce else 0, int(epoch))
+            _lib.call("gq_attach_delivery_counter", counter)
+
+        deliver()
+        return deliver
+
     def attach_delivery(self, plan):
         """Fused push: the next encode of `plan` into row `row()` also stores the record into the same
         row of every peer's block (or once through the multicast mapping) and then announces the new
-        epoch in every rank's flag array (its own included)."""
+        epoch in every rank's flag array (its own included).  Returns the function that re-attaches the
+        delivery for each launch of a multi-launch encode (FusedPlan.encode(delivery=...))."""
         self.epoch += 1
         local = self._addr(self.rank, self.rank)
         if self.mc_base:
@@ -124,17 +146,13 @@ class PeerRecords:
         else:
             deltas = [self._addr(r, self.rank) - local for r in range(self.world) if r != self.rank]
             mc = 0
-        ident = next((g for g in plan.groups if g.kind == "identity" and g.n), None)
-        ident_ptr = local + ident.raw_off if ident is not None else None
-        ident_bytes = (ident.n * 4 + 15) // 16 * 16 if ident is not None else 0
-        flags = (ctypes.c_void_p * self.world)(*[int(self._flag_ptrs[r]) + 4 * self.rank for r in range(self.world)])
-        _lib.call("gq_attach_remote_record", len(deltas), mc, (ctypes.c_int64 * len(deltas))(*deltas), ident_ptr,
-                  ident_bytes, ctypes.cast(flags, ctypes.c_void_p), self.world, self.epoch)
+        return self._delivery(plan, deltas, mc, list(range(self.world)), self.epoch, True)
 
     def attach_delivery_to(self, plan, targets, epoch, with_ident=True):
         """Ring hop: the next encode of `plan` into row `row()` also stores what it writes into the same
         row of the blocks of `targets` (all other ranks: once through the multicast mapping when there
-        is one) and then writes `epoch` into this rank's word of those ranks' flag arrays."""
+        is one) and then writes `epoch` into this rank's word of those ranks' flag arrays.  Returns the
+        re-attaching function, as attach_delivery does."""
         local = self._addr(self.rank, self.rank)
         everyone = len(targets) == self.world - 1
         if everyone and self.mc_base and self.world > 2:
@@ -145,20 +163,25 @@ class PeerRecords:
             deltas = [self._addr(r, self.rank) - local for r in targets]
             mc = 0
             flag_ranks = list(targets)
-        ident = next((g for g in plan.groups if g.kind == "identity" and g.n), None) if with_ident else None
-        ident_ptr = local + ident.raw_off if ident is not None else None
-        ident_bytes = (ident.n * 4 + 15) // 16 * 16 if ident is not None else 0
-        flags = (ctypes.c_void_p * len(flag_ranks))(*[int(self._flag_ptrs[r]) + 4 * self.rank for r in flag_ranks])
-        _lib.call("gq_attach_remote_record", len(deltas), mc, (ctypes.c_int64 * len(deltas))(*deltas), ident_ptr,
-                  ident_bytes, ctypes.cast(flags, ctypes.c_void_p), len(flag_ranks), int(epoch))
+        return self._delivery(plan, deltas, mc, flag_ranks, epoch, with_ident)
+
+    @staticmethod
+    def _wait(flags, n, epoch):
+        """Attach a wait now and return the function that attaches it again before each decode launch
+        (FusedPlan.decode(wait=...))."""
+        def wait():
+            _lib.call("gq_attach_peer_wait", flags, n, epoch)
+
+        wait()
+        return wait
 
     def attach_wait_for(self, src_rank, epoch):
         """Ring hop, receiving side: the next decode waits until `src_rank` has announced `epoch` here."""
-        _lib.call("gq_attach_peer_wait", int(self._flag_ptrs[self.rank]) + 4 * src_rank, 1, int(epoch))
+        return self._wait(int(self._flag_ptrs[self.rank]) + 4 * src_rank, 1, int(epoch))
 
     def attach_wait(self):
         """Fused push, receiving side: the next decode waits for every rank's flag of this epoch."""
-        _lib.call("gq_attach_peer_wait", int(self._flag_ptrs[self.rank]), self.world, self.epoch)
+        return self._wait(int(self._flag_ptrs[self.rank]), self.world, self.epoch)
 
     def barrier(self):
         self.epoch += 1

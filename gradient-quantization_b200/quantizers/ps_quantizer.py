@@ -48,7 +48,7 @@ class PSQuantizer(QuantizerBase):
         (args.p2p = False or GQ_P2P=0 turns it off)."""
         import torch.distributed as dist
         want = getattr(self.args, "p2p", True) and os.environ.get("GQ_P2P", "1") != "0"
-        ok = 1 if (want and self.world <= 8 and self.plan.supports_scattered()) else 0
+        ok = 1 if (want and self.world <= 8 and self.plan.supports_p2p()) else 0
         p2p = None
         err = None
         if ok:
@@ -74,6 +74,10 @@ class PSQuantizer(QuantizerBase):
             self.p2p_mode = os.environ.get("GQ_P2P_MODE", getattr(self.args, "p2p_mode", "push"))
             if self.p2p_mode not in ("push", "gather", "direct"):
                 raise _lib.GQError("unknown peer-to-peer mode %r" % (self.p2p_mode,))
+            if self.p2p_mode == "direct" and not self.plan.supports_scattered():
+                p2p.close()
+                raise _lib.GQError("peer-to-peer mode 'direct' (the decode reads the peers' records in place) supports "
+                                   "HSQ plans and identity tensors only; use 'push' or 'gather' for this codec")
             self.plan.records = p2p.records          # [2 * U, record_bytes]: row = parity * U + user
             # push + barrier launches disappear when the encode kernel delivers the record itself
             self.fused_push = (self.p2p_mode == "push" and os.environ.get("GQ_P2P_FUSED", "1") != "0"
@@ -146,10 +150,9 @@ class PSQuantizer(QuantizerBase):
         one process the record is decoded right after it is made (apply(), or the error feedback's
         decode), so the norm quantization moves into that decode (FusedPlan.encode(defer_levels=True));
         across processes the levels must exist before the record leaves the GPU."""
-        if self.fused_push:
-            self.p2p.attach_delivery(self.plan)
+        delivery = self.p2p.attach_delivery(self.plan) if self.fused_push else None
         defer = not self.distributed and self.plan.n_users == 1 and self.p2p is None
-        self.plan.encode(slot, src=src, uniforms=uniforms, rng_user=user, defer_levels=defer)
+        self.plan.encode(slot, src=src, uniforms=uniforms, rng_user=user, defer_levels=defer, delivery=delivery)
 
     def _scratch(self):
         if not hasattr(self, "_scratch_buf"):
@@ -183,22 +186,24 @@ class PSQuantizer(QuantizerBase):
         plan = self.plan
         out = plan.arena if out is None else out
         if self.p2p is not None:
+            wait = None
             if self.fused_push:
-                self.p2p.attach_wait()       # the decode kernel waits for every rank's delivery flag itself
+                wait = self.p2p.attach_wait()   # every decode kernel waits for every rank's delivery flag itself
             else:
                 if self.p2p_mode == "push":
                     self.p2p.push()
                 self.p2p.barrier()
                 if self.p2p_mode == "gather":
                     self.p2p.gather()
-            g = self.decode_exchanged(out)
+            g = self.decode_exchanged(out, wait=wait)
             self.p2p.advance()
             return g
         self.exchange()
         return plan.decode(mean=True, out=out)
 
-    def decode_exchanged(self, out=None):
-        """Decode-and-average all users' records of the current step (after the exchange)."""
+    def decode_exchanged(self, out=None, wait=None):
+        """Decode-and-average all users' records of the current step (after the exchange).  wait: the
+        fused push's re-attaching wait (PeerRecords.attach_wait), repeated before every decode launch."""
         plan = self.plan
         out = plan.arena if out is None else out
         if self.p2p is None:
@@ -206,7 +211,7 @@ class PSQuantizer(QuantizerBase):
         if self.p2p_mode == "direct":
             return plan.decode(n_users=self.world, mean=True, out=out, base_ptr=self.p2p.user0_record_ptr(),
                                user_offsets=self.p2p.user_offsets())
-        return plan.decode(first_user=self.p2p.row(0), n_users=self.world, mean=True, out=out)
+        return plan.decode(first_user=self.p2p.row(0), n_users=self.world, mean=True, out=out, wait=wait)
 
     # ------------------------------------------------------------------- apply
     def exchange(self):

@@ -46,12 +46,12 @@ class RingQuantizer(QuantizerBase):
         """Hops through peer-mapped memory: the encode kernel of rank r stores each stage of its record
         straight into rank r + 1's receive block and raises a flag the decode-accumulate kernel there
         waits on (the last rank: into every rank's block) -- the ps exchange's machinery, one target per
-        hop.  Needs the one-launch tcgen05 encode and the peer-to-peer decode (HSQ d = 8 / 16 / 32, K = 256,
-        FusedPlan.supports_fused_delivery and supports_scattered) on every rank."""
+        hop.  Needs a delivering encode and a plan the peer-to-peer exchange handles (FusedPlan.supports_p2p and
+        supports_fused_delivery: HSQ d = 8 / 16 / 32 with K = 256, sign, QSGD / TernGrad) on every rank."""
         import os
         import torch.distributed as dist
         want = getattr(self.args, "p2p", True) and os.environ.get("GQ_P2P", "1") != "0"
-        ok = 1 if (want and self.world <= 8 and self.plan.supports_scattered() and self.plan.supports_fused_delivery()) else 0
+        ok = 1 if (want and self.world <= 8 and self.plan.supports_p2p() and self.plan.supports_fused_delivery()) else 0
         p2p, err = None, None
         if ok:
             try:
@@ -121,11 +121,12 @@ class RingQuantizer(QuantizerBase):
                 # peer-to-peer hop: wait for the previous rank's flag inside the decode kernel, deliver this
                 # stage from inside the encode kernel (to the next rank; the last rank: to everybody)
                 if user != 0:
-                    self.p2p.attach_wait_for(user - 1, self._epoch(p))
-                    plan.decode(first_user=self.p2p.row(user - 1), n_users=1, mean=False, accumulate=True, out=buf, part=p)
+                    wait = self.p2p.attach_wait_for(user - 1, self._epoch(p))
+                    plan.decode(first_user=self.p2p.row(user - 1), n_users=1, mean=False, accumulate=True, out=buf, part=p,
+                                wait=wait)
                 targets = [user + 1] if user < last else [r for r in range(self.world) if r != user]
-                self.p2p.attach_delivery_to(plan, targets, self._epoch(p), with_ident=(p == 0))
-                plan.encode(self.p2p.row(), src=buf, uniforms=uniforms, rng_user=user, part=p)
+                delivery = self.p2p.attach_delivery_to(plan, targets, self._epoch(p), with_ident=(p == 0))
+                plan.encode(self.p2p.row(), src=buf, uniforms=uniforms, rng_user=user, part=p, delivery=delivery)
                 continue
             ranges = plan.part_byte_ranges(p)
             if user != 0:
@@ -161,9 +162,8 @@ class RingQuantizer(QuantizerBase):
         plan = self.plan
         last = self.args.num_users - 1
         if self.p2p is not None:
-            if self.rank != last:
-                self.p2p.attach_wait_for(last, self._epoch(self.parts - 1))
-            g = plan.decode(first_user=self.p2p.row(last), n_users=1, mean=False, out=out)
+            wait = self.p2p.attach_wait_for(last, self._epoch(self.parts - 1)) if self.rank != last else None
+            g = plan.decode(first_user=self.p2p.row(last), n_users=1, mean=False, out=out, wait=wait)
             self.p2p.advance()
             self._step += 1
             return g

@@ -329,17 +329,29 @@ int gq_peer_push(const void *src, void *const *dst_ptrs, size_t bytes, int n_dst
  * One multimem.st per 16 bytes is replicated by the switch to every rank (the sender included). */
 int gq_peer_push_multicast(const void *src, void *mc_dst, size_t bytes, gq_stream_t stream);
 
-/* Exchange fused into the codec kernels (default for HSQ d=16 K=256 on one NVSwitch node).
- * Sending side: the next gq_hsq_encode on this host thread also stores every finished section of
+/* Exchange fused into the codec kernels (default for HSQ at d = 8/16/32 with K = 256, sign and
+ * QSGD / TernGrad on one NVSwitch node).
+ * Sending side: the next encode call on this host thread also stores every finished section of
  * the record at (local address + delta[i]), i < n_remote -- the same record row in the peers'
  * receive blocks -- or once through an NVLS multicast mapping (multicast = 1, n_remote = 1),
  * mirrors the identity section [ident, ident + ident_bytes), and when the whole record is out stores
  * `epoch` (system-scope release) into flag_ptrs[0..n_flags): this rank's word in every rank's flag
- * array.  Receiving side: the next HSQ decode first waits until n_ranks words of local_flags have
- * reached `epoch`.  Together they replace gq_peer_push* + gq_peer_barrier (two launches per step)
+ * array.  n_flags == 0 delivers without announcing: an encode made of several calls (one per QSGD
+ * chunk size) attaches before each call and announces on the last one only.
+ * The delivering encodes are the one-launch tcgen05 HSQ encode (gq_hsq_encode: d = 8/16/32, K = 256,
+ * uint8 codes and levels), gq_sign_encode (packed output only), gq_sign_encode_t5 and gq_qsgd_encode
+ * on its one-launch chunked path (packed output only, 16-byte aligned, dim % 4 == 0, dim <= 2048) or
+ * its TernGrad path (explicit chunk boundaries).  Any other encode, gq_topk_select included, returns
+ * GQ_ERR_UNSUPPORTED and sends nothing; the pending delivery is cleared either way.  The sign and QSGD
+ * encodes send a section's last partial 32-bit word whole: their sections must be padded to 4 bytes.
+ * They also need gq_attach_delivery_counter: a zero-initialised 32-bit device word, not used by any
+ * other delivery at the same time, that their last CTA to arrive sets back to 0.
+ * Receiving side: the next HSQ, sign or QSGD decode first waits until n_ranks words of local_flags
+ * have reached `epoch`.  Together they replace gq_peer_push* + gq_peer_barrier (two launches per step)
  * of the exchange step of PSQuantizer (quantizers/ps_quantizer.py:44-48). */
 int gq_attach_remote_record(int n_remote, int multicast, const int64_t *delta, const void *ident,
                             int64_t ident_bytes, void *const *flag_ptrs, int n_flags, uint32_t epoch);
+int gq_attach_delivery_counter(void *counter);
 int gq_attach_peer_wait(const void *local_flags, int n_ranks, uint32_t epoch);
 
 /* ------------------------------------------------------------------------- */
